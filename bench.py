@@ -460,6 +460,9 @@ def run_b200(args):
     csz = np.empty(n, dtype=np.uint64)
     ctx._check(l.libdeflate_b200_memcpy_d2h(ctx.h, csz.ctypes.data, d_csz, 8 * n), "d2h")
     ctx.sync()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, l, n, chunk, cstride, csz, d_comp, d_out, d_aout, d_res,
+                     args.workload == "roundtrip")
     assert (csz > 0).all(), "a chunk did not fit its compress bound"
     # bit-exact byte comparison with the host originals on every 64th chunk
     samp = np.arange(0, n, 64)
@@ -665,6 +668,54 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
+DUMP_PER_CHUNK_BYTES = 12_000_000     # four float64 values per chunk listed
+DUMP_SAMPLE_BYTES = 48_000_000        # float32 bytes of the sampled chunks
+DUMP_SAMPLE_CHUNKS = 96
+
+
+def dump_outputs(out_dir, ctx, l, n, chunk, cstride, csz, d_comp, d_out, d_aout, d_res, compressed):
+    """What the last timed step handed back, as .npy files of float64 (per-chunk values) and float32 (bytes),
+    about 60 MB at most whatever the batch shape:
+      decompress_results, decompressed_sizes and, when the step compressed, compressed_sizes: one value per
+          chunk named in chunk_index -- every chunk, or a fixed, seeded sample once the batch is too large for
+          DUMP_PER_CHUNK_BYTES;
+      sample_decompressed and, when the step compressed, sample_compressed (the stream zero-padded to its slot):
+          the bytes of a fixed, seeded sample of chunks (sample_chunk_index), as many as DUMP_SAMPLE_BYTES holds
+          up to 96, and only the leading bytes of each when one chunk alone does not fit.
+    With --workload decompress the compressed streams are the reference's, an input of the step, so they are
+    not written.  The inputs are the same from run to run, so two builds compare file for file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+
+    def sample(count):
+        return np.arange(n) if count >= n else np.sort(rng.choice(n, count, replace=False))
+    res = np.empty(n, dtype=np.int32)
+    aout = np.empty(n, dtype=np.uint64)
+    ctx._check(l.libdeflate_b200_memcpy_d2h(ctx.h, res.ctypes.data, d_res, 4 * n), "d2h")
+    ctx._check(l.libdeflate_b200_memcpy_d2h(ctx.h, aout.ctypes.data, d_aout, 8 * n), "d2h")
+    per = sample(DUMP_PER_CHUNK_BYTES // (8 * 4))
+    arrays = {"chunk_index": per, "decompress_results": res[per], "decompressed_sizes": aout[per]}
+    row_bytes = 4 * (chunk + (cstride if compressed else 0))
+    idx = sample(max(1, min(DUMP_SAMPLE_CHUNKS, DUMP_SAMPLE_BYTES // row_bytes)))
+    cap = DUMP_SAMPLE_BYTES // (4 * len(idx) * (2 if compressed else 1))
+    out_len, comp_len = min(chunk, cap), min(cstride, cap)
+    out = np.empty((len(idx), out_len), dtype=np.uint8)
+    comp = np.zeros((len(idx), comp_len), dtype=np.uint8)
+    for k, i in enumerate(idx):
+        ctx._check(l.libdeflate_b200_memcpy_d2h(ctx.h, out[k].ctypes.data, d_out.slab + int(i) * chunk, out_len), "d2h")
+        if compressed:
+            ctx._check(l.libdeflate_b200_memcpy_d2h(ctx.h, comp[k].ctypes.data, d_comp.slab + int(i) * cstride,
+                                                    min(int(csz[i]), comp_len)), "d2h")
+    ctx.sync()
+    arrays.update(sample_chunk_index=idx, sample_decompressed=out)
+    if compressed:
+        arrays.update(compressed_sizes=csz[per], sample_compressed=comp)
+    for name, a in arrays.items():
+        a = a.astype(np.float32 if name.startswith("sample_") and name != "sample_chunk_index" else np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_e2e(args, ctx, l, ldb, pin_in, n, chunk, fmt, cstride, barrier, allmax, d_comp_ref, csz_ref):
     """Same metric through the host-buffer C-ABI calls a chunk-loop caller would make; pinned host memory on
     both sides.  The compressed side uses the PACKED forms (one buffer + offset table): the device packs the
@@ -833,6 +884,7 @@ def main():
     ap.add_argument("--overlap", action="store_true", help="e2e: also measure the two-host-thread form (compress of group g+1 over decompress of group g); "
                     "measured slower than the plain form (9.3 vs 10.06 GB/s, profiles/r02_e2e_overlap.md), hence off by default")
     ap.add_argument("--no-origin", action="store_true", help="N > 1: skip the single-origin (NCCL scatter/gather) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0's shard) to DIR/<name>.npy")
     args = ap.parse_args()
     LEVEL = args.level
     if args.warmup < 3:

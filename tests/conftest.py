@@ -91,22 +91,9 @@ def oracle():
     return Oracle()
 
 
-@pytest.fixture(scope="session")
-def reflib():
-    """The UNMODIFIED reference (oracle/_ref/libdeflate_ref.so) through the product's own
-    ctypes prototypes; skipped when it has not been built (it needs /root/reference)."""
-    import libdeflate_b200 as ldb
-    so = os.path.join(ROOT, "oracle", "_ref", "libdeflate_ref.so")
-    if not os.path.exists(so):
-        if os.path.isdir("/root/reference/lib"):
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], stdout=subprocess.DEVNULL)
-        else:
-            pytest.skip("oracle/_ref not built and /root/reference absent")
-    return ldb.Api(_load_ref(so))
-
-
 def _load_ref(so):
-    """The reference exports only the 21 classic symbols; attach just those prototypes."""
+    """The UNMODIFIED reference (oracle/_ref/libdeflate_ref.so, for tests/golden/make_fixtures.py): it
+    exports only the 21 classic symbols; attach just those prototypes."""
     import libdeflate_b200 as ldb
     lib = ctypes.CDLL(so)
     P, S, PS = ctypes.c_void_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)

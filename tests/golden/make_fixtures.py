@@ -1,7 +1,7 @@
 """Regenerates the committed golden fixtures.  Needs /root/reference (it runs the
 UNMODIFIED reference built into oracle/_ref/); the fixtures themselves travel with the repo.
 
-    python tests/golden/make_fixtures.py
+    python tests/golden/make_fixtures.py [ref_streams] [known_answers] [reference_answers]
 
 ref_streams.npz   : streams produced by the reference COMPRESSOR (levels 1/6/9/12, three
                     formats) with their plain texts -> pins bit-exact decompression.
@@ -9,6 +9,8 @@ known_answer.json : hand-assembled raw-DEFLATE streams in the spirit of the refe
                     programs/test_incomplete_codes.c, test_invalid_streams.c, test_overread.c
                     and test_slow_decompression.c, with the verdict and output bytes the
                     reference returned for them here.
+reference_answers.npz: the reference's answers for the inputs the tests compare with it
+                    (tests/reference_answers.py builds those inputs and reads the answers back).
 """
 import json
 import os
@@ -23,6 +25,8 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import corpus  # noqa: E402
 import deflate_asm as da  # noqa: E402
+import parity_checks as pc  # noqa: E402
+import reference_answers as ra  # noqa: E402
 import libdeflate_b200 as ldb  # noqa: E402
 from conftest import _load_ref  # noqa: E402
 
@@ -173,6 +177,32 @@ def known_answers():
         print("%-40s result=%d out=%d bytes" % (c["name"], c["result"], len(c["output"]) // 2))
 
 
+def reference_answers():
+    arrs = {}
+
+    def record(name, cases, answer):
+        arrs[name] = np.array([answer(c) for c in cases], dtype=np.uint64)
+        arrs[name + "_inputs"] = np.array(ra.inputs_digest(cases))
+
+    record("checksums", ra.checksum_cases(), lambda c: (ref.crc32(c[0], c[1]), ref.adler32(c[0], c[2])))
+    record("valid_streams", ra.valid_stream_cases(), lambda c: ra.outcome(ref.decompress(c[2], len(c[1]), c[0])))
+    record("fuzz", ra.fuzz_cases(), lambda c: ra.outcome(ref.decompress(c[1], c[2], c[0], c[3])))
+    record("gzip_header", pc.gzip_header_cases(), lambda c: ra.outcome(ref.decompress(c[1], len(c[0]), 2)))
+    names = ("deflate", "zlib", "gzip")
+    record("bound_and_stored", [(n, fmt) for n in ra.STORED_SIZES for fmt in (0, 1, 2)],
+           lambda c: (getattr(ref.l, "libdeflate_%s_compress_bound" % names[c[1]])(None, c[0]),
+                      ra.digest(ref.compress(corpus.rand(c[0], c[0]), 0, c[1]))))
+    chunks = ra.emu_deflate_chunks()
+    for name, levels, fmt in ra.EMU_DEFLATE_RUNS:
+        record("emu_deflate_" + name, chunks, lambda c: [len(ref.compress(c, lvl, fmt)) for lvl in levels])
+    record("levels_10_12", ra.chunks_1mib(), lambda c: [len(ref.compress(c, lvl, 0)) for lvl in ra.LEVELS_10_12])
+    import bench
+    for i, p in zip(ra.FULL_SIZE_INDICES, ra.full_size_plains(bench.load_synth())):
+        arrs["full_size_gzip6_%d" % i] = np.frombuffer(ref.compress(p, 6, 2), dtype=np.uint8)
+    np.savez_compressed(os.path.join(HERE, "reference_answers.npz"), **arrs)
+    print("reference_answers.npz:", {k: v.shape for k, v in arrs.items()})
+
+
 if __name__ == "__main__":
-    ref_streams()
-    known_answers()
+    for step in sys.argv[1:] or ["ref_streams", "known_answers", "reference_answers"]:
+        globals()[step]()

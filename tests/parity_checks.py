@@ -2,7 +2,8 @@
 
 Every check drives the SAME C-ABI entry points (`api`/`ctx` wrap either the product
 library on a B200 or the emulator build of the same kernel sources) and compares with
-the oracle (`orc`), with zlib, and -- when it is built -- with the unmodified reference.
+the oracle (`orc`), with zlib, and with what the unmodified reference answered for the same inputs
+(tests/reference_answers.py).
 """
 import random
 import zlib
@@ -40,9 +41,9 @@ def check_checksum_batch(ctx, orc, n_chunks=67, max_len=70000, seed=4):
     assert ctx.checksum_batch_host(bufs, "adler32") == [zlib.adler32(b) for b in bufs]
 
 
-def make_valid_streams(sizes=(0, 1, 100, 5000, 65536), levels=(1, 6, 9), ref=None):
-    """(format, plain, stream) triples from zlib (independent producer) and, if available,
-    from the reference compressor itself (SURVEY.md section 8c parity definition)."""
+def make_valid_streams(sizes=(0, 1, 100, 5000, 65536), levels=(1, 6, 9)):
+    """(format, plain, stream) triples from zlib (independent producer); the reference compressor's own
+    streams are reference_answers.fixture_streams() (SURVEY.md section 8c parity definition)."""
     out = []
     for n in sizes:
         for name, plain in corpus.all_classes(n, n + 5).items():
@@ -51,9 +52,6 @@ def make_valid_streams(sizes=(0, 1, 100, 5000, 65536), levels=(1, 6, 9), ref=Non
                     out.append((fmt, plain, corpus.zlib_raw(plain, lv, zlib.Z_DEFAULT_STRATEGY, wb)))
                 out.append((fmt, plain, corpus.zlib_raw(plain, 6, zlib.Z_FIXED, wb)))
                 out.append((fmt, plain, corpus.zlib_raw(plain, 0, zlib.Z_DEFAULT_STRATEGY, wb)))
-                if ref is not None:
-                    for lv in (1, 6, 12):
-                        out.append((fmt, plain, ref.compress(plain, lv, fmt)))
     return out
 
 
@@ -224,11 +222,9 @@ def gzip_member(plain, flg, level=6, extra=b"EXTRA-field", name=b"file name.txt"
     return hdr + body + struct.pack("<II", zlib.crc32(plain), len(plain) & 0xffffffff), len(hdr)
 
 
-def check_gzip_optional_fields(ctx, orc, ref=None):
-    """ref: lib/gzip_decompress.c:66-98 -- FEXTRA / FNAME / FCOMMENT / FHCRC (and FTEXT) in every combination are
-    skipped with bounds checks; reserved FLG bits, truncation inside any field, a missing NUL and a header that leaves
-    fewer than 8 bytes for the trailer are BAD_DATA.  Verdicts, actual_in and bytes must equal the oracle's (and the
-    unmodified reference's, when it is built)."""
+def gzip_header_cases():
+    """(plain, gzip stream): every combination of the optional header fields, cut inside each of them, reserved
+    FLG bits, a missing NUL, empty and long fields."""
     plain = corpus.text(3000, 7)
     cases = []
     for flg in range(32):
@@ -248,14 +244,25 @@ def check_gzip_optional_fields(ctx, orc, ref=None):
     z, _ = gzip_member(plain, 4, extra=b"q" * 300)
     cases.append(z)
     cases.append(z[:12 + 100])                                      # cut inside FEXTRA
-    got = ctx.decompress_batch_host(cases, [len(plain)] * len(cases), 2)
+    return [(plain, z) for z in cases]
+
+
+def check_gzip_optional_fields(ctx, orc, ref_answers=None):
+    """ref: lib/gzip_decompress.c:66-98 -- FEXTRA / FNAME / FCOMMENT / FHCRC (and FTEXT) in every combination are
+    skipped with bounds checks; reserved FLG bits, truncation inside any field, a missing NUL and a header that leaves
+    fewer than 8 bytes for the trailer are BAD_DATA.  Verdicts, actual_in and bytes must equal the oracle's (and,
+    given `ref_answers`, the unmodified reference's answers for gzip_header_cases())."""
+    import reference_answers as ra
+    cases = gzip_header_cases()
+    plain = cases[0][0]
+    got = ctx.decompress_batch_host([z for _, z in cases], [len(plain)] * len(cases), 2)
     seen = set()
-    for z, g in zip(cases, got):
+    for k, ((_, z), g) in enumerate(zip(cases, got)):
         o = orc.decompress(z, len(plain), 2)
         assert g[0] == o[0] and (o[0] != 0 or g == o), ("gzip header case", z[:24].hex(), g[0], o[0], g[2:], o[2:])
-        if ref is not None:
-            r = ref.decompress(z, len(plain), 2)
-            assert r[0] == o[0] and (o[0] != 0 or r == o), ("oracle vs reference", z[:24].hex(), r[0], o[0])
+        if ref_answers is not None:
+            r = ref_answers[k]
+            assert r[0] == o[0] and (o[0] != 0 or r == ra.outcome(o)), ("oracle vs reference", z[:24].hex(), r[0], o[0])
         seen.add(o[0])
     assert seen >= {0, 1}, seen
 
@@ -309,12 +316,13 @@ def check_decompress_fuzz(ctx, checker, cases):
     return n_by_verdict
 
 
-def check_compress_round_trip(ctx, orc, chunks, levels=(1, 6, 9), fmts=(0, 1, 2), ref=None, max_ratio_vs_ref=None):
+def check_compress_round_trip(ctx, orc, chunks, levels=(1, 6, 9), fmts=(0, 1, 2)):
     """Compressed bytes are not contractual (libdeflate.h:76-83); what is: the stream inflates
     back to the input with the oracle AND zlib, it fits *_compress_bound(), an exactly sized
-    output buffer works and one byte less returns 0."""
+    output buffer works and one byte less returns 0.  Returns the compressed sizes, format by
+    format, level by level, chunk by chunk."""
     wbits = {0: -15, 1: 15, 2: 31}
-    stats = []
+    sizes = []
     for fmt in fmts:
         for lvl in levels:
             zs = ctx.compress_batch_host(chunks, lvl, fmt)
@@ -324,18 +332,13 @@ def check_compress_round_trip(ctx, orc, chunks, levels=(1, 6, 9), fmts=(0, 1, 2)
                 r = orc.decompress(z, len(c), fmt)
                 assert r[0] == 0 and r[1] == c and r[2] == len(z), ("oracle cannot inflate it", fmt, lvl, len(c))
                 assert zlib.decompress(z, wbits[fmt]) == c
-                if ref is not None:
-                    stats.append((lvl, len(c), len(z), len(ref.compress(c, lvl, fmt))))
+                sizes.append(len(z))
             # exact fit and one-byte-short (same streams are deterministic)
             exact = [ctx.compress_batch_host([c], lvl, fmt, out_avail=len(z))[0] for c, z in list(zip(chunks, zs))[:3]]
             assert all(e == z for e, z in zip(exact, zs)), ("exact-size buffer failed", fmt, lvl)
             short = [ctx.compress_batch_host([c], lvl, fmt, out_avail=len(z) - 1)[0] for c, z in list(zip(chunks, zs))[:3]]
             assert all(s is None for s in short), ("short buffer did not return 0", fmt, lvl)
-    if ref is not None and max_ratio_vs_ref is not None:
-        ours = sum(s[2] for s in stats)
-        theirs = sum(s[3] for s in stats)
-        assert ours <= theirs * max_ratio_vs_ref, ("ratio regression", ours, theirs)
-    return stats
+    return sizes
 
 
 def check_host_pipeline(library, ctx, n=2304, chunk=4096):

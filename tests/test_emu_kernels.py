@@ -5,6 +5,7 @@ ever the nvcc build, exercised by test_gpu_parity.py under `-m gpu`.
 """
 import pytest
 import parity_checks as pc
+import reference_answers as ra
 
 
 def test_checksum_kernels_emulated(emu_api, oracle):
@@ -15,13 +16,13 @@ def test_checksum_batch_emulated(emu_ctx, oracle):
     pc.check_checksum_batch(emu_ctx, oracle, n_chunks=40, max_len=20000)
 
 
-def test_inflate_valid_streams_emulated(emu_ctx, oracle, reflib):
-    streams = pc.make_valid_streams(sizes=(0, 1, 100, 5000, 40000), levels=(1, 6), ref=reflib)
+def test_inflate_valid_streams_emulated(emu_ctx, oracle):
+    streams = pc.make_valid_streams(sizes=(0, 1, 100, 5000, 40000), levels=(1, 6)) + ra.fixture_streams()
     pc.check_decompress_valid(emu_ctx, oracle, streams)
 
 
-def test_gzip_optional_header_fields_emulated(emu_ctx, oracle, reflib):
-    pc.check_gzip_optional_fields(emu_ctx, oracle, reflib)
+def test_gzip_optional_header_fields_emulated(emu_ctx, oracle):
+    pc.check_gzip_optional_fields(emu_ctx, oracle, ra.answers("gzip_header", pc.gzip_header_cases()))
 
 
 def test_inflate_truncation_and_space_sweep_emulated(emu_ctx, oracle):
@@ -41,12 +42,12 @@ def test_inflate_fuzz_emulated(emu_ctx, oracle):
     assert set(v) >= {0, 1, 3}, v
 
 
-def test_deflate_round_trip_emulated(emu_ctx, oracle, reflib):
-    import corpus
-    chunks = [b"", b"a", corpus.text(56, 1), corpus.text(3000, 2), corpus.pattern(9000), corpus.rand(6000, 3),
-              corpus.zeros(70000), corpus.mixed(40000, 4), corpus.text(65536, 5), corpus.text(100000, 6)]
-    pc.check_compress_round_trip(emu_ctx, oracle, chunks, levels=(0, 1, 6, 12), fmts=(0,), ref=reflib, max_ratio_vs_ref=1.10)
-    pc.check_compress_round_trip(emu_ctx, oracle, chunks, levels=(6,), fmts=(2,), ref=reflib, max_ratio_vs_ref=1.10)
+def test_deflate_round_trip_emulated(emu_ctx, oracle):
+    chunks = ra.emu_deflate_chunks()
+    for name, levels, fmt in ra.EMU_DEFLATE_RUNS:
+        ours = sum(pc.check_compress_round_trip(emu_ctx, oracle, chunks, levels=levels, fmts=(fmt,)))
+        theirs = sum(sum(r) for r in ra.answers("emu_deflate_" + name, chunks))      # the reference's sizes
+        assert ours <= theirs * 1.10, ("ratio regression", name, ours, theirs)
     pc.check_compress_round_trip(emu_ctx, oracle, chunks[:6], levels=(3, 9), fmts=(1,))
 
 

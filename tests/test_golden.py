@@ -4,21 +4,14 @@ import json
 import os
 import random
 
-import numpy as np
-
 import deflate_asm as da
+import reference_answers as ra
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def _known():
     return json.load(open(os.path.join(HERE, "golden", "known_answer.json")))
-
-
-def _ref_streams():
-    fx = np.load(os.path.join(HERE, "golden", "ref_streams.npz"))
-    names = sorted(k[:-2] for k in fx.files if k.endswith("_z"))
-    return [(int(n[1]), fx[n + "_p"].tobytes(), fx[n + "_z"].tobytes()) for n in names]
 
 
 def test_oracle_known_answers(oracle):
@@ -30,7 +23,7 @@ def test_oracle_known_answers(oracle):
 
 
 def test_oracle_inflates_reference_compressor_output(oracle):
-    for fmt, plain, z in _ref_streams():
+    for fmt, plain, z in ra.fixture_streams():
         r = oracle.decompress(z, len(plain), fmt)
         assert r[0] == 0 and r[1] == plain and r[2] == len(z)
 
@@ -45,7 +38,7 @@ def test_kernel_logic_known_answers_emulated(emu_ctx):
 
 
 def test_kernel_logic_reference_streams_emulated(emu_ctx):
-    streams = _ref_streams()
+    streams = ra.fixture_streams()
     for fmt in (0, 1, 2):
         sel = [s for s in streams if s[0] == fmt]
         got = emu_ctx.decompress_batch_host([s[2] for s in sel], [len(s[1]) for s in sel], fmt)

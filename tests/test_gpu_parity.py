@@ -4,6 +4,7 @@ import ctypes
 import glob
 import os
 import subprocess
+import sys
 import zlib
 
 import numpy as np
@@ -11,16 +12,30 @@ import pytest
 
 import corpus
 import parity_checks as pc
+import reference_answers as ra
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 pytestmark = pytest.mark.gpu
 
 
+NATIVE_ONLY = """
+import libdeflate_b200 as ldb
+assert ldb.lib().libdeflate_b200_device_count() >= 1
+maps = open("/proc/self/maps").read()
+assert "libdeflate_b200.so" in maps and "libdeflate_b200_emu" not in maps
+"""
+
+
 def test_native_library_is_loaded():
     import libdeflate_b200 as ldb
     assert ldb.lib().libdeflate_b200_device_count() >= 1
-    maps = open("/proc/self/maps").read()
-    assert "libdeflate_b200.so" in maps and "libdeflate_b200_emu" not in maps
+    assert ldb.lib()._name == ldb.LIB_PATH and os.path.basename(ldb.LIB_PATH) == "libdeflate_b200.so"
+    assert "libdeflate_b200.so" in open("/proc/self/maps").read()
+    # the package on its own loads the nvcc build and never the emulator build; checked in a fresh
+    # interpreter, since the CPU tests of the same session load the emulator build into this one
+    r = subprocess.run([sys.executable] + (["-s"] if sys.flags.no_user_site else []) + ["-c", NATIVE_ONLY], cwd=ROOT,
+                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, timeout=300)
+    assert r.returncode == 0, r.stdout.decode()[-2000:]
 
 
 def test_checksums_single_call(gpu_api, oracle):
@@ -81,25 +96,19 @@ def test_gzip_optional_header_fields(gpu_ctx, oracle):
 def test_compress_1mib_chunks_levels_10_12(gpu_ctx, oracle):
     """BASELINE configs[3] shape: 1 MiB chunks through the near-optimal levels (the ring is crossed 16 times, the
     DP segment logic 512 times per chunk): round trip, bound, and the ratio next to the reference's."""
-    chunks = [corpus.text(1 << 20, 11), corpus.mixed(1 << 20, 12), corpus.rand(1 << 20, 13), corpus.zeros(1 << 20)]
-    ref_so = os.path.join(ROOT, "oracle", "_ref", "libdeflate_ref.so")
-    ref = None
-    if os.path.exists(ref_so):
-        import libdeflate_b200 as ldb
-        from conftest import _load_ref
-        ref = ldb.Api(_load_ref(ref_so))
-    for lvl in (10, 12):
+    chunks = ra.chunks_1mib()
+    ref_sizes = ra.answers("levels_10_12", chunks)
+    for k, lvl in enumerate(ra.LEVELS_10_12):
         zs = gpu_ctx.compress_batch_host(chunks, lvl, 0)
-        for c, z in zip(chunks, zs):
+        for c, z, rs in zip(chunks, zs, ref_sizes):
             assert z is not None and len(z) <= oracle.l.oracle_compress_bound(0, len(c))
             assert zlib.decompress(z, -15) == c
             r = oracle.decompress(z, len(c), 0)
             assert r[0] == 0 and r[1] == c and r[2] == len(z)
-            if ref is not None:
-                # (measured: 13 % behind at level 10 on this very repetitive text -- no length-3 matches, 2 cost passes;
-                # the guard is a regression fence, the numbers are in DESIGN.md)
-                # + 1 KiB: our blocks end every 32 KiB, 32 block headers per MiB show on inputs that shrink to ~1 KB (zeros: 1838 vs 1070 B)
-                assert len(z) <= 1.16 * len(ref.compress(c, lvl, 0)) + 1024, ("ratio vs reference", lvl, len(z), len(ref.compress(c, lvl, 0)))
+            # (measured: 13 % behind at level 10 on this very repetitive text -- no length-3 matches, 2 cost passes;
+            # the guard is a regression fence, the numbers are in DESIGN.md)
+            # + 1 KiB: our blocks end every 32 KiB, 32 block headers per MiB show on inputs that shrink to ~1 KB (zeros: 1838 vs 1070 B)
+            assert len(z) <= 1.16 * rs[k] + 1024, ("ratio vs reference", lvl, len(z), rs[k])
 
 
 def test_two_contexts_two_host_threads(gpu_ctx):
@@ -247,25 +256,19 @@ def test_pipelined_host_path(gpu_ctx):
 
 
 def test_full_size_property_round_trip(gpu_ctx):
-    """BASELINE-sized chunks: 4096 x 64 KiB synthetic text, reference streams in,
+    """BASELINE-sized batch: 4096 x 64 KiB chunks of the robustness mix T/P/S/R/Z/M, the reference's
+    level-6 gzip streams in (the committed streams of 21 distinct chunks, cycled through the batch),
     checksum-of-checksums out (size-independent property)."""
     import bench
-    synth = bench.load_synth()
-    cpub = bench.load_cpub()
-    if cpub is None:
-        pytest.skip("oracle/_ref not prebuilt")
-    n, chunk = 4096, 65536
-    buf = (ctypes.c_uint8 * (n * chunk))()
-    synth.synth_fill(buf, chunk, 0, n, 6, 8)      # robustness mix T/P/S/R/Z/M
-    tc, td, total, streams = bench.cpu_roundtrip(cpub, 2, 6, buf, chunk, n, bench.host_threads(), want_streams=True)
-    comp, stride, sizes = streams
-    raw = bytes(comp)
-    zs = [raw[i * stride:i * stride + sizes[i]] for i in range(n)]
-    got = gpu_ctx.decompress_batch_host(zs, chunk, 2)
-    plain = bytes(buf)
+    plains = ra.full_size_plains(bench.load_synth())
+    fx = ra.load()
+    streams = [fx["full_size_gzip6_%d" % i].tobytes() for i in ra.FULL_SIZE_INDICES]
+    n, chunk = 4096, ra.FULL_SIZE_CHUNK
+    got = gpu_ctx.decompress_batch_host([streams[i % len(streams)] for i in range(n)], chunk, 2)
+    crcs = [zlib.crc32(p) for p in plains]
     for i, g in enumerate(got):
         assert g[0] == 0 and g[3] == chunk
-        assert zlib.crc32(g[1]) == zlib.crc32(plain[i * chunk:(i + 1) * chunk])
+        assert zlib.crc32(g[1]) == crcs[i % len(crcs)]
 
 
 def test_reference_test_programs_against_our_library():
