@@ -47,8 +47,21 @@
 #define LZ_PASS      16384			// positions matched + parsed per pass
 #define LZ_BLOCK_PASSES 2			// passes per DEFLATE block (32 KiB of input)
 #define LZ_NWIN      (LZ_PASS / 32)
-#define LZ_NSL_BITS  (LZ_WARPS >= 32 ? 5 : 4)	// hash slices of the insertion = linking warps
-#define LZ_NSL       (1 << LZ_NSL_BITS)
+// Levels 1-9 run two warp groups: the search group (warps [0, LZ_A_WARPS)) loads, inserts and searches
+// pass after pass; the encode group (the other warps) parses each searched pass and encodes the blocks,
+// one pass behind.  -DLZ_PIPELINE=0 runs both halves on the whole CTA, one after the other (the serial
+// schedule, which levels 10-12 always use).  Both schedules produce the same stream.
+#ifndef LZ_PIPELINE
+#define LZ_PIPELINE  1
+#endif
+#ifndef LZ_A_WARPS
+#define LZ_A_WARPS   22
+#endif
+#define LZ_B_WARPS   (LZ_WARPS - LZ_A_WARPS)
+#define LZ_BAR_A     1			// named barriers: the search group,
+#define LZ_BAR_B     2			//   the encode group,
+#define LZ_BAR_FULL  3			//   "pass s searched" (3 + s % 2, search group arrives, encode group waits)
+#define LZ_BAR_EMPTY 5			//   "pass s released" (5 + s % 2, encode group arrives, search group waits)
 #ifndef LZ_QUANTUM
 #define LZ_QUANTUM   0			// > 0: chain steps per loop trip of the resumable search (experiment)
 #endif
@@ -60,8 +73,8 @@
 #define LZ_MAX_DIST  (LZ_WIN - LZ_LOOKAHEAD)	// the oldest LOOKAHEAD bytes of the window are overwritten
 #define LZ_TOKCAP    (LZ_BLOCK_PASSES * LZ_PASS + 64)
 #define LZ_STAGE_WORDS 2048			// 8 KiB emission staging
-#define LZ_TPT         (LZ_THREADS > 512 ? 1 : 2)	// tokens per thread per emission round
-#define LZ_EMIT_ROUND  (LZ_THREADS * LZ_TPT)	// tokens per emission round (<= 48 bits each, <= 1536 words)
+#define LZ_TPT_MAX     3			// tokens per thread per emission round: LZ_THREADS / (threads encoding),
+					// so a round is <= 1024 tokens of <= 48 bits (<= 1536 staging words)
 
 // shared memory layout
 #define LZ_SM_RING   0
@@ -79,7 +92,11 @@
 #define LZ_SM_LENS   (LZ_SM_FREQ + 4 * 320)			// u8[320]
 #define LZ_SM_CODES  (LZ_SM_LENS + 320)				// u16[320]
 #define LZ_SM_VARS   (LZ_SM_CODES + 2 * 320)			// misc scalars, mbarrier
-#define LZ_SM_BYTES  (LZ_SM_VARS + 256)
+#define LZ_SM_CMAT   (LZ_SM_VARS + 256)				// u32[A_WARPS * 16 + 32] insertion counts of the search group
+#define LZ_SM_BYTES  (LZ_SM_CMAT + 4 * (LZ_A_WARPS * 16 + 32))	//   (pipelined; region R is the encode group's then)
+static_assert(LZ_SM_BYTES <= 227 * 1024, "shared memory of one CTA");
+static_assert(LZ_A_WARPS >= 16 && LZ_B_WARPS * 32 >= 320 && LZ_THREADS / (LZ_B_WARPS * 32) <= LZ_TPT_MAX,
+	      "search group: >= one warp per hash slice; encode group: one thread per litlen+offset symbol");
 
 // per-CTA global scratch (L2 resident): per-position results of the current pass + tokens
 #define LZ_BLOCK_POS (LZ_BLOCK_PASSES * LZ_PASS)		// positions per block
@@ -90,6 +107,7 @@
 #define LZ_GS_COST   (LZ_GS_TOK + 4 * LZ_TOKCAP)		// u32[BLOCK_POS + 320]   (levels 10-12)
 #define LZ_GS_MLIST  (LZ_GS_COST + 4 * (LZ_BLOCK_POS + 320))	// u32[BLOCK_POS * K]     (levels 10-12)
 #define LZ_GS_BYTES  (LZ_GS_MLIST + 4 * LZ_BLOCK_POS * LZ_OPT_K)
+#define LZ_GS_EXIT   LZ_GS_MLIST				// u16[PASS] parse exits (pipelined; levels 1-9 keep no match lists)
 #define LZ_FAR4_DIST  1024				// text-like input: a 4-byte match further away than this is coded as literals
 #define LZ_COST_INF  0x3fffffu				// fits the 23-bit cost field of the DP reduction key
 
@@ -114,7 +132,51 @@ struct lz_vars {
 	u32 obit_lo, obit_hi;	// output bit position (64-bit)
 	u32 pre_lens_packed[3];
 	u32 tma_phase;
+	u32 slot_chunk[2], slot_b0[2], slot_min_len[2], slot_far4[2];	// pass s handed to the encode group: slot s % 2
 };
+static_assert(sizeof(lz_vars) <= 256, "LZ_SM_VARS");
+#define LZ_NO_CHUNK  0xffffffffu		// slot_chunk of the pass after the last one
+
+// A warp group: thread / warp index inside the group, its size, and its barrier (0: the whole CTA).
+struct lz_grp {
+	u32 t, w, nt, nw, bar;
+};
+#ifdef LDB_EMU
+// bar.sync / bar.arrive for the emulator build: a barrier completes when 'nthreads' threads have arrived.
+// The emulator runs all threads of a block on one host thread (and one block at a time on it), and a
+// completed barrier is back at 0 arrivals, so per-host-thread state needs no reset between blocks.
+inline void lz_emu_named_barrier(u32 id, u32 nthreads, bool wait)
+{
+	static thread_local struct { u32 arrived, gen; } bars[16];
+	auto &b = bars[id & 15];
+	const u32 gen = b.gen;
+	if (++b.arrived == nthreads) {
+		b.arrived = 0;
+		b.gen++;
+		emu::tl_block->spins = 0;
+	} else if (wait) {
+		while (b.gen == gen) emu::yield();
+	}
+}
+#endif
+__device__ __forceinline__ void lz_bar_sync(u32 id, u32 nthreads)
+{
+#ifdef LDB_EMU
+	if (id == 0) __syncthreads();
+	else lz_emu_named_barrier(id, nthreads, true);
+#else
+	asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+#endif
+}
+__device__ __forceinline__ void lz_bar_arrive(u32 id, u32 nthreads)
+{
+#ifdef LDB_EMU
+	lz_emu_named_barrier(id, nthreads, false);
+#else
+	asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+#endif
+}
+__device__ __forceinline__ void lz_sync(const lz_grp &gp) { lz_bar_sync(gp.bar, gp.nt); }
 
 struct lz_params {
 	int depth, nice, lazy;
@@ -179,16 +241,16 @@ __device__ __forceinline__ u32 lz_ld8(const u8 *ring, u32 pos) { return ring[pos
 __device__ __forceinline__ u32 lz_hash(u32 v) { return (v * 0x1E35A7BDu) >> (32 - LZ_HASH_BITS); }	// ref: matchfinder_common.h:168-172
 
 // ---- TMA bulk load of one segment into the ring -------------------------------------
-__device__ __forceinline__ void lz_load_segment(u8 *sm, lz_vars *v, const u8 *in, u32 from, u32 to)
+__device__ __forceinline__ void lz_load_segment(u8 *sm, lz_vars *v, const u8 *in, u32 from, u32 to, const lz_grp &gp)
 {
 	u8 *ring = sm + LZ_SM_RING;
 	u32 len = to - from;
 	u32 bulk = (((uintptr_t)(in + from) & 15) == 0) ? (len & ~15u) : 0;
-	__syncthreads();	// every earlier generic-proxy access to the slots being overwritten is done
+	lz_sync(gp);	// every earlier generic-proxy access to the slots being overwritten is done
 #ifndef LDB_EMU
 	if (bulk) {
 		u32 mbar = (u32)__cvta_generic_to_shared(&v->mbar);
-		if (threadIdx.x == 0) {
+		if (gp.t == 0) {
 			u32 dst = (u32)__cvta_generic_to_shared(ring + (from & (LZ_RING - 1)));
 			asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 			asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bulk) : "memory");
@@ -203,12 +265,12 @@ __device__ __forceinline__ void lz_load_segment(u8 *sm, lz_vars *v, const u8 *in
 		}
 	}
 #else
-	for (u32 i = threadIdx.x; i < bulk; i += LZ_THREADS) ring[(from + i) & (LZ_RING - 1)] = in[from + i];
+	for (u32 i = gp.t; i < bulk; i += gp.nt) ring[(from + i) & (LZ_RING - 1)] = in[from + i];
 #endif
-	for (u32 i = bulk + threadIdx.x; i < len; i += LZ_THREADS) ring[(from + i) & (LZ_RING - 1)] = in[from + i];
-	__syncthreads();
-	if (bulk && threadIdx.x == 0) v->tma_phase ^= 1;
-	__syncthreads();
+	for (u32 i = bulk + gp.t; i < len; i += gp.nt) ring[(from + i) & (LZ_RING - 1)] = in[from + i];
+	lz_sync(gp);
+	if (bulk && gp.t == 0) v->tma_phase ^= 1;
+	lz_sync(gp);
 }
 
 // ---- length / offset slot helpers (Appendix A; ref: deflate_compress.c:237-308) ------
@@ -256,14 +318,14 @@ __device__ __forceinline__ void lz_stage_or(u32 *stage, u32 rel_bit, u64 bits, u
 }
 
 // Writes staging words [0, nwords) to the output at word index 'first_word'; all threads.
-__device__ __forceinline__ void lz_flush_words(const lz_out &o, const u32 *stage, u64 first_word, u32 nwords)
+__device__ __forceinline__ void lz_flush_words(const lz_out &o, const u32 *stage, u64 first_word, u32 nwords, const lz_grp &gp)
 {
 	if ((((uintptr_t)o.out) & 3) == 0) {
 		u32 *dst = (u32 *)o.out + first_word;
-		for (u32 i = threadIdx.x; i < nwords; i += LZ_THREADS) dst[i] = stage[i];
+		for (u32 i = gp.t; i < nwords; i += gp.nt) dst[i] = stage[i];
 	} else {
 		u8 *dst = o.out + first_word * 4;
-		for (u32 i = threadIdx.x; i < nwords * 4; i += LZ_THREADS) dst[i] = (u8)(stage[i >> 2] >> (8 * (i & 3)));
+		for (u32 i = gp.t; i < nwords * 4; i += gp.nt) dst[i] = (u8)(stage[i >> 2] >> (8 * (i & 3)));
 	}
 }
 
@@ -322,7 +384,7 @@ __device__ __forceinline__ void lz_gen_codes_serial(const u8 *lens, u32 nsyms, u
 // the compiler may read the clock before the barrier wait, so a phase in which thread 0 finishes early
 // is under-counted and the wait shows up in the next one: read 'search phase' + 'parse e1' together)
 __device__ unsigned long long ldb_lz_timing[16];
-#define LZ_T(k) do { if (tid == 0) { long long t_ = clock64(); tacc[k] += t_ - tlast; tlast = t_; } } while (0)
+#define LZ_T(k) do { if (tlead) { long long t_ = clock64(); tacc[k] += t_ - tlast; tlast = t_; } } while (0)
 #else
 #define LZ_T(k) do { } while (0)
 #endif
@@ -343,7 +405,7 @@ __device__ __forceinline__ u32 lz_same_key_mask(u32 key, bool valid)
 
 // ---- ordered hash-chain insertion of one pass by the whole CTA -------------------------------
 // Chains must link every position to the previous one with the same hash, so insertion is ordered
-// -- but only within a hash value.  The head table is cut into LZ_NSL (16 or 32) slices by the top hash bits
+// -- but only within a hash value.  The head table is cut into NSL (16 or 32) slices by the top hash bits
 // and the pass is split stably by slice (a multisplit), after which one warp per slice links it:
 //  (1) warp w hashes its contiguous range of tiles, parks each hash in the position's own next[]
 //      slot (dead until the link is written) and counts its positions per slice;
@@ -354,62 +416,68 @@ __device__ __forceinline__ u32 lz_same_key_mask(u32 key, bool valid)
 //      the same-slice lane mask): every list ends up sorted by position;
 //  (4) warp s links list s, 32 entries at a time: predecessors inside the batch come from
 //      the same-hash lane mask, the others from head[].  Same links as a serial insertion.
+template <u32 NW>	// warps of the group (gp.nw)
 __device__ __forceinline__ void lz_insert_pass_par(const u8 *ring, u16 *head, u16 *nextt, u32 *cmat,
-						   u32 b0, u32 pend, u32 n, u32 tid, u32 lane, u32 warp
+						   u32 b0, u32 pend, u32 n, const lz_grp &gp, u32 lane
 #ifdef LZ_TIMING
 						   , long long *tacc, long long &tlast
 #endif
 						   )
 {
-	static_assert(LZ_WARPS >= LZ_NSL && (LZ_WARPS * LZ_NSL + 2 * LZ_NSL) * 4 <= 8192, "one linking warp per slice");
-	u32 *sbase = cmat + LZ_WARPS * LZ_NSL, *stot = sbase + LZ_NSL;
+	constexpr u32 NSL_BITS = NW >= 32 ? 5 : 4, NSL = 1u << NSL_BITS;	// hash slices = linking warps
+	static_assert(NW >= NSL && (NW * NSL + 2 * NSL) * 4 <= 8192, "one linking warp per slice");
+	const u32 tid = gp.t, warp = gp.w;
+#ifdef LZ_TIMING
+	const bool tlead = tid == 0;
+#endif
+	u32 *sbase = cmat + NW * NSL, *stot = sbase + NSL;
 	const u32 lt = (1u << lane) - 1;
 	const u32 LB = (b0 + LZ_PASS) & 0xffff;
-	const u32 ntiles = (pend - b0 + 31) >> 5, tpw = (ntiles + LZ_WARPS - 1) / LZ_WARPS;
+	const u32 ntiles = (pend - b0 + 31) >> 5, tpw = (ntiles + NW - 1) / NW;
 	const u32 r0 = b0 + warp * tpw * 32;
 	const u32 r1 = r0 + tpw * 32 < pend ? r0 + tpw * 32 : pend;
-	for (u32 i = tid; i < LZ_WARPS * LZ_NSL + 2 * LZ_NSL; i += LZ_THREADS) cmat[i] = 0;
-	__syncthreads();
+	for (u32 i = tid; i < NW * NSL + 2 * NSL; i += 32 * NW) cmat[i] = 0;
+	lz_sync(gp);
 	for (u32 p = r0 + lane; p < r1; p += 32) {
 		const u32 hv = p + 4 <= n ? lz_hash(lz_ld32(ring, p)) : 0xffffu;
 		nextt[p & 0xffff] = (u16)hv;
-		if (hv != 0xffffu) atomicAdd(&cmat[warp * LZ_NSL + (hv >> (LZ_HASH_BITS - LZ_NSL_BITS))], 1u);
+		if (hv != 0xffffu) atomicAdd(&cmat[warp * NSL + (hv >> (LZ_HASH_BITS - NSL_BITS))], 1u);
 	}
-	__syncthreads();
+	lz_sync(gp);
 	LZ_T(12);	// insertion: hashing
 	if (warp == 0) {
 		u32 run = 0;
-		if (lane < LZ_NSL)
-			for (u32 w = 0; w < LZ_WARPS; w++) {
-				const u32 c = cmat[w * LZ_NSL + lane];
-				cmat[w * LZ_NSL + lane] = run;
+		if (lane < NSL)
+			for (u32 w = 0; w < NW; w++) {
+				const u32 c = cmat[w * NSL + lane];
+				cmat[w * NSL + lane] = run;
 				run += c;
 			}
 		u32 incl = run;
-		for (int o2 = 1; o2 < LZ_NSL; o2 <<= 1) {
+		for (int o2 = 1; o2 < NSL; o2 <<= 1) {
 			const u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
 			if (lane >= (u32)o2) incl += t;
 		}
-		if (lane < LZ_NSL) { sbase[lane] = incl - run; stot[lane] = run; }
+		if (lane < NSL) { sbase[lane] = incl - run; stot[lane] = run; }
 	}
-	__syncthreads();
+	lz_sync(gp);
 	for (u32 t = 0; t < tpw; t++) {
 		const u32 p = r0 + 32 * t + lane;
 		const u32 hv = p < r1 ? nextt[p & 0xffff] : 0xffffu;
 		const bool valid = hv != 0xffffu;
-		const u32 sl = hv >> (LZ_HASH_BITS - LZ_NSL_BITS);
-		const u32 m = lz_same_key_mask<LZ_NSL_BITS>(sl, valid);
-		const u32 cur = valid ? cmat[warp * LZ_NSL + sl] : 0;
+		const u32 sl = hv >> (LZ_HASH_BITS - NSL_BITS);
+		const u32 m = lz_same_key_mask<NSL_BITS>(sl, valid);
+		const u32 cur = valid ? cmat[warp * NSL + sl] : 0;
 		__syncwarp();
 		if (valid) {
 			nextt[LB + sbase[sl] + cur + __popc(m & lt)] = (u16)p;
-			if ((m & lt) == 0) cmat[warp * LZ_NSL + sl] = cur + __popc(m);
+			if ((m & lt) == 0) cmat[warp * NSL + sl] = cur + __popc(m);
 		}
 		__syncwarp();
 	}
-	__syncthreads();
+	lz_sync(gp);
 	LZ_T(13);	// insertion: slice lists
-	if (warp < LZ_NSL) {
+	if (warp < NSL) {
 		const u32 cnt = stot[warp];
 		const u16 *mylist = nextt + LB + sbase[warp];
 		u32 p16n = lane < cnt ? mylist[lane] : 0;
@@ -423,7 +491,7 @@ __device__ __forceinline__ void lz_insert_pass_par(const u8 *ring, u16 *head, u1
 				hn = nextt[p16n];
 			}
 			const u32 old_head = valid ? head[h] : 0;
-			const u32 m = lz_same_key_mask<LZ_HASH_BITS - LZ_NSL_BITS>(h, valid);	// (the slice bits are equal anyway)
+			const u32 m = lz_same_key_mask<LZ_HASH_BITS - NSL_BITS>(h, valid);	// (the slice bits are equal anyway)
 			const u32 below = m & lt;
 			const u32 prev = __shfl_sync(LDB_FULL_MASK, p16, below ? 31 - __clz(below) : 0);
 			if (valid) {
@@ -433,7 +501,7 @@ __device__ __forceinline__ void lz_insert_pass_par(const u8 *ring, u16 *head, u1
 			__syncwarp();
 		}
 	}
-	__syncthreads();
+	lz_sync(gp);
 }
 
 // ---- one chain search (ref: hc_matchfinder.h:182-338) ------------------------------------------
@@ -683,10 +751,10 @@ __device__ void lz_dp_segment(const u8 *ring, const u32 *mlist, u32 *costg, u32 
 // Here blocks end on pass boundaries, so the test runs once per pass, on the bytes of the pass that
 // would join the block: lz_observe() counts their classes (all threads), lz_should_end_block()
 // applies the reference's integer arithmetic to the two histograms.
-__device__ __forceinline__ void lz_observe(const u8 *ring, u32 from, u32 to, u32 *obs, u32 tid, u32 lane)
+__device__ __forceinline__ void lz_observe(const u8 *ring, u32 from, u32 to, u32 *obs, const lz_grp &gp, u32 lane)
 {
 	// 16 bytes per thread and round; class counts in 8 packed byte fields, reduced per warp
-	for (u32 wbase = from + 512 * (tid >> 5); wbase < to; wbase += 16 * LZ_THREADS) {	// warp-uniform trip count
+	for (u32 wbase = from + 512 * gp.w; wbase < to; wbase += 16 * gp.nt) {	// warp-uniform trip count
 		const u32 base = wbase + 16 * lane;
 		const uint4 q = *(const uint4 *)(ring + (base & (LZ_RING - 1)));	// from is 16 KiB aligned
 		const u32 w[4] = {q.x, q.y, q.z, q.w};
@@ -756,11 +824,17 @@ ldb_deflate_lz_kernel(ldb_deflate_args a)
 	u8 *costtab = sm + LZ_SM_ITEMS;	// lit[256] len[259] off[32] bit costs of the DP (the items region is free then)
 
 	const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const lz_params P = lz_level_params(a.level);
+	// the two warp groups (levels 1-9), or the whole CTA for both halves (serial schedule)
+	const bool pipe = LZ_PIPELINE && !P.opt_iters;
+	const bool in_a = !pipe || warp < LZ_A_WARPS;
+	const lz_grp gA = pipe ? lz_grp{tid, warp, 32 * LZ_A_WARPS, LZ_A_WARPS, LZ_BAR_A} : lz_grp{tid, warp, LZ_THREADS, LZ_WARPS, 0};
+	const lz_grp gB = pipe ? lz_grp{tid - 32 * LZ_A_WARPS, warp - LZ_A_WARPS, 32 * LZ_B_WARPS, LZ_B_WARPS, LZ_BAR_B} : gA;
 #ifdef LZ_TIMING
 	long long tacc[16] = {};
 	long long tlast = clock64();
+	const bool tlead = (in_a ? gA : gB).t == 0;	// one clock per group
 #endif
-	const lz_params P = lz_level_params(a.level);
 
 	if (tid == 0) {
 		v->tma_phase = 0;
@@ -772,57 +846,36 @@ ldb_deflate_lz_kernel(ldb_deflate_args a)
 	}
 	__syncthreads();
 
-	for (;;) {
-		if (tid == 0) v->chunk = atomicAdd(a.work_counter, 1u);
-		__syncthreads();
-		const size_t c = v->chunk;
-		__syncthreads();
-		if (c >= a.n) break;
+	const u32 overhead = a.format == LDB_FMT_GZIP ? 18 : (a.format == LDB_FMT_ZLIB ? 6 : 0);
+	const u32 trailer = a.format == LDB_FMT_GZIP ? 8 : (a.format == LDB_FMT_ZLIB ? 4 : 0);
+	const u32 hdr_bytes = overhead - trailer;
+	// encode-group state of the chunk being encoded
+	size_t c = 0, n64 = 0;
+	u32 n = 0;
+	const u8 *in = nullptr;
+	lz_out o;
+	o.out = nullptr; o.avail = 0; o.obit = 0;
+	u32 cmin_len = 4, cfar4 = LZ_WIN;	// the chunk's minimum match length and far-4 distance (from the search group)
+	u32 block_begin = 0;
+	u32 block_entry = 0;	// position of the first token of the current block
+	u32 pass_in_block = 0;
+	// res holds two passes: pass s (numbered across chunks) at (s % 2) * PASS.  Levels 10-12 index it by
+	// the pass in the block instead: their min-cost path covers the whole block.
+	auto res_off = [&](u32 s) -> u32 { return (P.opt_iters ? pass_in_block : (s & 1)) * LZ_PASS; };
 
-		const u8 *in = (const u8 *)a.in_ptrs[c];
-		const size_t n64 = a.in_nbytes[c];
-		lz_out o;
+	auto chunk_begin = [&](const lz_grp &gp, size_t cc, u32 min_len, u32 far4) {
+		c = cc;
+		in = (const u8 *)a.in_ptrs[c];
+		n64 = a.in_nbytes[c];
+		n = (u32)n64;
 		o.out = (u8 *)a.out_ptrs[c];
 		o.avail = a.out_avail[c];
-		o.obit = 0;
-		const u32 overhead = a.format == LDB_FMT_GZIP ? 18 : (a.format == LDB_FMT_ZLIB ? 6 : 0);
-		const u32 trailer = a.format == LDB_FMT_GZIP ? 8 : (a.format == LDB_FMT_ZLIB ? 4 : 0);
-		const u32 hdr_bytes = overhead - trailer;
-
-		// ---- tiny inputs and oversize chunks take the stored path (ref: deflate_compress.c:4041-4043)
-		const bool passthrough = n64 <= (size_t)(55 - 4 * a.level) || n64 > 0x7fff0000u;
-		bool fits = !(overhead && o.avail <= overhead);
-		if (passthrough || !fits) {
-			const size_t nblocks = n64 ? (n64 + 65534) / 65535 : 1;
-			fits = fits && (n64 + 5 * nblocks <= o.avail - overhead);
-			if (!fits) {
-				if (tid == 0) a.out_nbytes[c] = 0;
-				continue;
-			}
-			if (tid == 0) def_write_header(o.out, a.format, a.level);
-			u8 *dst = o.out + hdr_bytes;
-			for (size_t b = 0; b < nblocks; b++) {
-				size_t off = b * 65535;
-				u32 len = (u32)(n64 - off > 65535 ? 65535 : n64 - off);
-				if (tid == 0) {
-					dst[0] = (b + 1 == nblocks) ? 1 : 0;
-					dst[1] = (u8)len; dst[2] = (u8)(len >> 8);
-					dst[3] = (u8)~len; dst[4] = (u8)(~len >> 8);
-				}
-				for (u32 i = tid; i < len; i += LZ_THREADS) dst[5 + i] = in[off + i];
-				dst += 5 + len;
-			}
-			if (tid == 0) {
-				u32 t = def_write_trailer(dst, a.format, a.checksums ? a.checksums[c] : 0, n64);
-				a.out_nbytes[c] = (size_t)(dst - o.out) + t;
-			}
-			continue;
-		}
-		const u32 n = (u32)n64;
-
-		// ---- per-chunk init ---------------------------------------------------------------
-		for (u32 i = tid; i < (1u << LZ_HASH_BITS) / 2; i += LZ_THREADS) ((u32 *)head)[i] = 0xffffffffu;
-		if (tid == 0) {
+		cmin_len = min_len;
+		cfar4 = far4;
+		block_begin = 0;
+		block_entry = 0;
+		pass_in_block = 0;
+		if (gp.t == 0) {
 			v->failed = 0;
 			v->parse_entry = 0;
 			v->tok_count = 0;
@@ -835,1039 +888,1172 @@ ldb_deflate_lz_kernel(ldb_deflate_args a)
 			for (u32 i = whole; i < hdr_bytes; i++) cw |= (u32)h[i] << (8 * (i - whole));
 			v->carry = cw;
 		}
-		for (u32 i = tid; i < 320; i += LZ_THREADS) freq[i] = 0;
+		if (gp.t < 8) v->obs_blk[gp.t] = 0;
+		for (u32 i = gp.t; i < 320; i += gp.nt) freq[i] = 0;
 		o.obit = (u64)hdr_bytes * 8;
-		__syncthreads();
+		lz_sync(gp);
+		// byte classes of the first pass (the block-split test compares the next pass against them)
+		lz_observe(ring, 0, n < LZ_PASS ? n : LZ_PASS, v->obs_blk, gp, lane);
+		lz_sync(gp);
+	};
 
-		// ---- exact parallel parse of one pass (positions [pb0, ppend), results at res[aoff + i]).
-		// forced: the DP already decided (flag set on matches); otherwise the lazy rule decides.
-		// exitt: 16 Ki u16 of scratch in shared memory -- the link slots of the first pass that is not
-		// inserted yet (dead, see lz_insert_pass_par)
-		auto parse_pass = [&](const u32 pb0, const u32 ppend, const u32 aoff, const bool forced, u16 *exitt) {
-			// (e1) per-window decisions + "exit position for every entry lane" by pointer jumping
-			const u32 nwin = (ppend - pb0 + 31) >> 5;
-			// (the per-position results live in L2: the loads run two windows ahead of their use)
-			const u32 min_len = v->min_len, far4 = v->far4_dist;
-			auto e1_load = [&](u32 w, u32 &x0, u32 &x1, u32 &x2) {
-				x0 = 0; x1 = 0; x2 = 0;
-				if (w < nwin) {
-					const u32 i = w * 32 + lane;
-					if (pb0 + i < ppend) x0 = res[aoff + i];
-					if (lane == 31 && pb0 + i + 1 < ppend) x1 = res[aoff + i + 1];	// (the others get it by shuffle)
-					if (lane == 31 && P.lazy == 2 && pb0 + i + 2 < ppend) x2 = res[aoff + i + 2];
-				}
-			};
-			u32 cW0, cW1, cW2, nW0, nW1, nW2;
-			e1_load(warp, cW0, cW1, cW2);
-			e1_load(warp + LZ_WARPS, nW0, nW1, nW2);
-			for (u32 w = warp; w < nwin; w += LZ_WARPS) {
-				u32 i = w * 32 + lane;
-				u32 p = pb0 + i;
-				const u32 W0 = cW0, nb = __shfl_down_sync(LDB_FULL_MASK, W0, 1), W1 = lane == 31 ? cW1 : nb;
-				const u32 nb2 = __shfl_down_sync(LDB_FULL_MASK, W1, 1), W2 = lane == 31 ? cW2 : nb2;	// two ahead (lazy2)
-				const u32 L0 = W0 & 0xffff, O0 = ((W0 >> 16) & 0x7fff) + 1, L1 = W1 & 0xffff, O1 = ((W1 >> 16) & 0x7fff) + 1;
-				cW0 = nW0; cW1 = nW1; cW2 = nW2;
-				e1_load(w + 2 * LZ_WARPS, nW0, nW1, nW2);
-				// (a shortest-possible match at a long distance costs more bits than its literals: the
-				// reference's rule for length 3 beyond 8 KiB, deflate_compress.c:2666-2668, restated for our
-				// minimum length 4)
-				bool is_match = forced ? ((L0 >= 3) && p < ppend) : (L0 >= min_len && p < ppend && !(L0 == 4 && O0 > far4));
-				if (!forced && is_match && P.lazy && p + 1 < ppend) {
-					// ref: deflate_compress.c:2722-2725 -- prefer the next position's match if clearly better
-					if (L1 >= L0 && L0 < (u32)P.nice &&
-					    4 * ((int)L1 - (int)L0) + ((int)(31 - __clz((int)O0)) - (int)(31 - __clz((int)O1))) > 2)
-						is_match = false;
-					if (P.lazy == 2 && is_match && p + 2 < ppend) {
-						// ref: deflate_compress.c:2757-2760 -- or the one after it, by a wider margin
-						const u32 L2 = W2 & 0xffff, O2 = ((W2 >> 16) & 0x7fff) + 1;
-						if (L2 >= L0 && L0 < (u32)P.nice &&
-						    4 * ((int)L2 - (int)L0) + ((int)(31 - __clz((int)O0)) - (int)(31 - __clz((int)O2))) > 6)
-							is_match = false;
-					}
-				}
-				u32 step = is_match ? L0 : 1;
-				// decision flag in the top bit; the neighbour that reads res[aoff + i] for its lazy test
-				// masks it off, and it only reads -- the flag is published after this warp's reads
-				__syncwarp();
-				if (is_match && !forced) res[aoff + i] = L0 | (((O0 - 1) | 0x8000u) << 16);
-				u32 j = lane + step;
-#pragma unroll
-				for (int k = 0; k < 5; k++) {
-					u32 t = __shfl_sync(LDB_FULL_MASK, j, j & 31);
-					if (j < 32) j = t;
-				}
-				if (p < ppend) exitt[i] = (u16)j;
+	// ---- exact parallel parse of one pass (positions [pb0, ppend), results at res[aoff + i]).
+	// forced: the DP already decided (flag set on matches); otherwise the lazy rule decides.
+	// exitt: 16 Ki u16 of scratch in shared memory -- the link slots of the first pass that is not
+	// inserted yet (dead, see lz_insert_pass_par)
+	auto parse_pass = [&](const lz_grp &gp, const u32 pb0, const u32 ppend, const u32 aoff, const bool forced, u16 *exitt) {
+		// (e1) per-window decisions + "exit position for every entry lane" by pointer jumping
+		const u32 nwin = (ppend - pb0 + 31) >> 5;
+		// (the per-position results live in L2: the loads run two windows ahead of their use)
+		const u32 min_len = cmin_len, far4 = cfar4;
+		auto e1_load = [&](u32 w, u32 &x0, u32 &x1, u32 &x2) {
+			x0 = 0; x1 = 0; x2 = 0;
+			if (w < nwin) {
+				const u32 i = w * 32 + lane;
+				if (pb0 + i < ppend) x0 = res[aoff + i];
+				if (lane == 31 && pb0 + i + 1 < ppend) x1 = res[aoff + i + 1];	// (the others get it by shuffle)
+				if (lane == 31 && P.lazy == 2 && pb0 + i + 2 < ppend) x2 = res[aoff + i + 2];
 			}
-			__syncthreads();
-			LZ_T(8);
-			// (e2) chain the windows.  A serial walk over all windows costs ~300 cycles per window on
-			// one warp, so it is split: (a) every warp composes the exits of ITS group of windows for
-			// all 32 possible entry lanes of the group's first window (per-lane shuffles), (b) warp 0
-			// chains the 16 groups, (c) every warp re-walks its group along the one real trajectory and
-			// records the entry lane of each window.
-			{
-				const u32 G = (nwin + LZ_WARPS - 1) / LZ_WARPS;		// windows per group
-				const u32 wg0 = warp * G;				// first window of my group
-				const u32 gstart = wg0 * 32;				// pass-relative position
-				// (a) exits of the group for entries gstart + lane
-				{
-					u32 pos = gstart + lane;
-					for (u32 k0 = 0; k0 < G; k0 += 8) {
-						u32 ex[8];
-#pragma unroll
-						for (int k = 0; k < 8; k++) {
-							u32 w = wg0 + k0 + k;
-							u32 i = w * 32 + lane;
-							ex[k] = (k0 + k < G && w < nwin && pb0 + i < ppend) ? exitt[i] : (lane + 1);
-						}
-#pragma unroll
-						for (int k = 0; k < 8; k++) {
-							u32 w = wg0 + k0 + k;
-							u32 x = __shfl_sync(LDB_FULL_MASK, ex[k], pos & 31);
-							if (k0 + k < G && w < nwin && (pos >> 5) == w) pos = (w << 5) + x;
-						}
-					}
-					gexit[warp * 32 + lane] = (u16)(pos > 0xffff ? 0xffff : pos);
+		};
+		u32 cW0, cW1, cW2, nW0, nW1, nW2;
+		e1_load(gp.w, cW0, cW1, cW2);
+		e1_load(gp.w + gp.nw, nW0, nW1, nW2);
+		for (u32 w = gp.w; w < nwin; w += gp.nw) {
+			u32 i = w * 32 + lane;
+			u32 p = pb0 + i;
+			const u32 W0 = cW0, nb = __shfl_down_sync(LDB_FULL_MASK, W0, 1), W1 = lane == 31 ? cW1 : nb;
+			const u32 nb2 = __shfl_down_sync(LDB_FULL_MASK, W1, 1), W2 = lane == 31 ? cW2 : nb2;	// two ahead (lazy2)
+			const u32 L0 = W0 & 0xffff, O0 = ((W0 >> 16) & 0x7fff) + 1, L1 = W1 & 0xffff, O1 = ((W1 >> 16) & 0x7fff) + 1;
+			cW0 = nW0; cW1 = nW1; cW2 = nW2;
+			e1_load(w + 2 * gp.nw, nW0, nW1, nW2);
+			// (a shortest-possible match at a long distance costs more bits than its literals: the
+			// reference's rule for length 3 beyond 8 KiB, deflate_compress.c:2666-2668, restated for our
+			// minimum length 4)
+			bool is_match = forced ? ((L0 >= 3) && p < ppend) : (L0 >= min_len && p < ppend && !(L0 == 4 && O0 > far4));
+			if (!forced && is_match && P.lazy && p + 1 < ppend) {
+				// ref: deflate_compress.c:2722-2725 -- prefer the next position's match if clearly better
+				if (L1 >= L0 && L0 < (u32)P.nice &&
+				    4 * ((int)L1 - (int)L0) + ((int)(31 - __clz((int)O0)) - (int)(31 - __clz((int)O1))) > 2)
+					is_match = false;
+				if (P.lazy == 2 && is_match && p + 2 < ppend) {
+					// ref: deflate_compress.c:2757-2760 -- or the one after it, by a wider margin
+					const u32 L2 = W2 & 0xffff, O2 = ((W2 >> 16) & 0x7fff) + 1;
+					if (L2 >= L0 && L0 < (u32)P.nice &&
+					    4 * ((int)L2 - (int)L0) + ((int)(31 - __clz((int)O0)) - (int)(31 - __clz((int)O2))) > 6)
+						is_match = false;
 				}
-				__syncthreads();
-				// (b) chain the groups (warp 0, all lanes redundantly; lane 0 publishes)
-				if (warp == 0) {
-					u32 e = v->parse_entry - pb0;	// pass-relative
-					for (u32 g = 0; g < LZ_WARPS; g++) {
-						const u32 gs = g * G * 32, ge = (g + 1) * G * 32;
-						u32 ent = 0xffffffffu;
-						if (e < ge && gs < (nwin << 5) && pb0 + e < ppend) {
-							ent = e;
-							if (e < gs + 32) {
-								e = gexit[g * 32 + (e - gs)];
-							} else {
-								// entered past the group's first window (a long match jumped in): walk it
-								for (u32 w = e >> 5; w < (g + 1) * G && w < nwin; w++) {
-									if ((e >> 5) == w) {
-										u32 i = w * 32 + (e & 31);
-										u32 x = pb0 + i < ppend ? exitt[i] : ((e & 31) + 1);
-										e = (w << 5) + x;
-									}
+			}
+			u32 step = is_match ? L0 : 1;
+			// decision flag in the top bit; the neighbour that reads res[aoff + i] for its lazy test
+			// masks it off, and it only reads -- the flag is published after this warp's reads
+			__syncwarp();
+			if (is_match && !forced) res[aoff + i] = L0 | (((O0 - 1) | 0x8000u) << 16);
+			u32 j = lane + step;
+#pragma unroll
+			for (int k = 0; k < 5; k++) {
+				u32 t = __shfl_sync(LDB_FULL_MASK, j, j & 31);
+				if (j < 32) j = t;
+			}
+			if (p < ppend) exitt[i] = (u16)j;
+		}
+		lz_sync(gp);
+		LZ_T(8);
+		// (e2) chain the windows.  A serial walk over all windows costs ~300 cycles per window on
+		// one warp, so it is split: (a) every warp composes the exits of ITS group of windows for
+		// all 32 possible entry lanes of the group's first window (per-lane shuffles), (b) warp 0
+		// chains the groups, (c) every warp re-walks its group along the one real trajectory and
+		// records the entry lane of each window.
+		{
+			const u32 G = (nwin + gp.nw - 1) / gp.nw;		// windows per group
+			const u32 wg0 = gp.w * G;				// first window of my group
+			const u32 gstart = wg0 * 32;				// pass-relative position
+			// (a) exits of the group for entries gstart + lane
+			{
+				u32 pos = gstart + lane;
+				for (u32 k0 = 0; k0 < G; k0 += 8) {
+					u32 ex[8];
+#pragma unroll
+					for (int k = 0; k < 8; k++) {
+						u32 w = wg0 + k0 + k;
+						u32 i = w * 32 + lane;
+						ex[k] = (k0 + k < G && w < nwin && pb0 + i < ppend) ? exitt[i] : (lane + 1);
+					}
+#pragma unroll
+					for (int k = 0; k < 8; k++) {
+						u32 w = wg0 + k0 + k;
+						u32 x = __shfl_sync(LDB_FULL_MASK, ex[k], pos & 31);
+						if (k0 + k < G && w < nwin && (pos >> 5) == w) pos = (w << 5) + x;
+					}
+				}
+				gexit[gp.w * 32 + lane] = (u16)(pos > 0xffff ? 0xffff : pos);
+			}
+			lz_sync(gp);
+			// (b) chain the groups (warp 0, all lanes redundantly; lane 0 publishes)
+			if (gp.w == 0) {
+				u32 e = v->parse_entry - pb0;	// pass-relative
+				for (u32 g = 0; g < gp.nw; g++) {
+					const u32 gs = g * G * 32, ge = (g + 1) * G * 32;
+					u32 ent = 0xffffffffu;
+					if (e < ge && gs < (nwin << 5) && pb0 + e < ppend) {
+						ent = e;
+						if (e < gs + 32) {
+							e = gexit[g * 32 + (e - gs)];
+						} else {
+							// entered past the group's first window (a long match jumped in): walk it
+							for (u32 w = e >> 5; w < (g + 1) * G && w < nwin; w++) {
+								if ((e >> 5) == w) {
+									u32 i = w * 32 + (e & 31);
+									u32 x = pb0 + i < ppend ? exitt[i] : ((e & 31) + 1);
+									e = (w << 5) + x;
 								}
 							}
 						}
-						if (lane == 0) gentry[g] = ent;
 					}
-					u32 fin = pb0 + e;
-					if (fin < ppend) fin = ppend;
-					__syncwarp();	// every lane has read parse_entry (racecheck: read/write by different lanes)
-					if (lane == 0) v->parse_entry = fin;
+					if (lane == 0) gentry[g] = ent;
 				}
-				__syncthreads();
-				// (c) entry lane of every window of my group along the real trajectory
-				{
-					u32 pos = gentry[warp];
-					for (u32 k0 = 0; k0 < G; k0 += 8) {
-						u32 ex[8];
+				u32 fin = pb0 + e;
+				if (fin < ppend) fin = ppend;
+				__syncwarp();	// every lane has read parse_entry (racecheck: read/write by different lanes)
+				if (lane == 0) v->parse_entry = fin;
+			}
+			lz_sync(gp);
+			// (c) entry lane of every window of my group along the real trajectory
+			{
+				u32 pos = gentry[gp.w];
+				for (u32 k0 = 0; k0 < G; k0 += 8) {
+					u32 ex[8];
 #pragma unroll
-						for (int k = 0; k < 8; k++) {
-							u32 w = wg0 + k0 + k;
-							u32 i = w * 32 + lane;
-							ex[k] = (k0 + k < G && w < nwin && pb0 + i < ppend) ? exitt[i] : (lane + 1);
+					for (int k = 0; k < 8; k++) {
+						u32 w = wg0 + k0 + k;
+						u32 i = w * 32 + lane;
+						ex[k] = (k0 + k < G && w < nwin && pb0 + i < ppend) ? exitt[i] : (lane + 1);
+					}
+#pragma unroll
+					for (int k = 0; k < 8; k++) {
+						u32 w = wg0 + k0 + k;
+						if (k0 + k < G && w < nwin) {
+							bool inside = pos != 0xffffffffu && (pos >> 5) == w && pb0 + pos < ppend;
+							u32 x = __shfl_sync(LDB_FULL_MASK, ex[k], pos & 31);
+							if (lane == 0) entryt[w] = inside ? (u8)(pos & 31) : 0xff;
+							if (inside) pos = (w << 5) + x;
 						}
-#pragma unroll
-						for (int k = 0; k < 8; k++) {
-							u32 w = wg0 + k0 + k;
-							if (k0 + k < G && w < nwin) {
-								bool inside = pos != 0xffffffffu && (pos >> 5) == w && pb0 + pos < ppend;
-								u32 x = __shfl_sync(LDB_FULL_MASK, ex[k], pos & 31);
-								if (lane == 0) entryt[w] = inside ? (u8)(pos & 31) : 0xff;
-								if (inside) pos = (w << 5) + x;
-							}
-						}
 					}
 				}
 			}
-			__syncthreads();
-			LZ_T(9);
-			// (e3) visited sets per window (the loads of the next window are issued first)
-			auto e3_load = [&](u32 w, u32 &e, u32 &x) {
-				e = 0xff; x = 0;
-				if (w < nwin) {
-					const u32 i = w * 32 + lane;
-					e = entryt[w];
-					if (e != 0xff && pb0 + i < ppend) x = res[aoff + i];
-				}
-			};
-			u32 e3_e, e3_w, e3_ne, e3_nw;
-			e3_load(warp, e3_e, e3_w);
-			e3_load(warp + LZ_WARPS, e3_ne, e3_nw);
-			for (u32 w = warp; w < nwin; w += LZ_WARPS) {
-				const u32 e = e3_e, rw = e3_w;
-				e3_e = e3_ne; e3_w = e3_nw;
-				e3_load(w + 2 * LZ_WARPS, e3_ne, e3_nw);
-				u32 V = 0;
-				if (e != 0xff) {
-					u32 step = (rw & 0x80000000u) ? (rw & 0xffff) : 1;
-					u32 j = lane + step;
-					u32 jk[5];
-#pragma unroll
-					for (int k = 0; k < 5; k++) {
-						jk[k] = j;
-						u32 t = __shfl_sync(LDB_FULL_MASK, j, j & 31);
-						if (j < 32) j = t;
-					}
-					V = 1u << e;
-#pragma unroll
-					for (int k = 4; k >= 0; k--) {
-						u32 contrib = (((V >> lane) & 1) && jk[k] < 32) ? (1u << jk[k]) : 0;
-						V |= __reduce_or_sync(LDB_FULL_MASK, contrib);
-					}
-					// positions at or beyond the end of the pass are not tokens of this block
-					const u32 wbase = pb0 + w * 32;
-					if (wbase + 32 > ppend) V &= ppend > wbase ? ((1u << (ppend - wbase)) - 1) : 0;
-				}
-				if (lane == 0) vis[w] = V;
+		}
+		lz_sync(gp);
+		LZ_T(9);
+		// (e3) visited sets per window (the loads of the next window are issued first)
+		auto e3_load = [&](u32 w, u32 &e, u32 &x) {
+			e = 0xff; x = 0;
+			if (w < nwin) {
+				const u32 i = w * 32 + lane;
+				e = entryt[w];
+				if (e != 0xff && pb0 + i < ppend) x = res[aoff + i];
 			}
-			__syncthreads();
-			LZ_T(10);
-			// (e4) token offsets (exclusive scan over windows) by warp 0
-			if (warp == 0) {
-				u32 run = 0;
-				for (u32 w0 = 0; w0 < nwin; w0 += 32) {
-					u32 w = w0 + lane;
-					u32 c = w < nwin ? (u32)__popc(vis[w]) : 0;
-					u32 incl = c;
-					for (int o2 = 1; o2 < 32; o2 <<= 1) {
-						u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
-						if (lane >= (u32)o2) incl += t;
-					}
-					if (w < nwin) tokoff[w] = run + incl - c;
-					run += __shfl_sync(LDB_FULL_MASK, incl, 31);
-				}
-				if (lane == 0) tokoff[LZ_NWIN] = run;
-			}
-			__syncthreads();
-			LZ_T(11);
-			// (e5) emit tokens + histograms
-			const u32 tbase = v->tok_count;
-			auto e5_load = [&](u32 w, u32 &V, u32 &x) {
-				V = 0; x = 0;
-				if (w < nwin) {
-					V = vis[w];
-					if ((V >> lane) & 1) x = res[aoff + w * 32 + lane];
-				}
-			};
-			u32 e5_V, e5_w, e5_nV, e5_nw;
-			e5_load(warp, e5_V, e5_w);
-			e5_load(warp + LZ_WARPS, e5_nV, e5_nw);
-			for (u32 w = warp; w < nwin; w += LZ_WARPS) {
-				const u32 V = e5_V, ro = e5_w >> 16;
-				const u32 len = e5_w & 0xffff;
-				e5_V = e5_nV; e5_w = e5_nw;
-				e5_load(w + 2 * LZ_WARPS, e5_nV, e5_nw);
-				if (!V) continue;
-				u32 i = w * 32 + lane;
-				if ((V >> lane) & 1) {
-					u32 idx = tbase + tokoff[w] + __popc(V & ((1u << lane) - 1));
-					u32 off = (ro & 0x7fff) + 1;
-					// (a match that does not fit the data would be a bug upstream; never emit one)
-					if ((ro & 0x8000) && len >= 3 && len <= 258 && off <= pb0 + i && pb0 + i + len <= n) {
-						tokbuf[idx] = 0x80000000u | ((len - 3) << 15) | (off - 1);
-						atomicAdd(&freq[257 + lz_len_slot(len)], 1u);
-						atomicAdd(&freq[288 + lz_off_slot(off)], 1u);
-					} else {
-						u32 bv = lz_ld8(ring, pb0 + i);
-						tokbuf[idx] = bv;
-						atomicAdd(&freq[bv], 1u);
-					}
-				}
-			}
-			__syncthreads();
-			if (tid == 0) v->tok_count = tbase + tokoff[LZ_NWIN];
-			__syncthreads();
 		};
-
-		// ---- Huffman codes from freq[] -> lens[], codes[] (all threads)
-		// CTA-wide exclusive scan (all threads must call it); escan[0..64] is the scratch
-		auto cta_excl_scan = [&](u32 x, u32 &total) -> u32 {
-			u32 incl = x;
-			for (int o2 = 1; o2 < 32; o2 <<= 1) {
-				u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
-				if (lane >= (u32)o2) incl += t;
+		u32 e3_e, e3_w, e3_ne, e3_nw;
+		e3_load(gp.w, e3_e, e3_w);
+		e3_load(gp.w + gp.nw, e3_ne, e3_nw);
+		for (u32 w = gp.w; w < nwin; w += gp.nw) {
+			const u32 e = e3_e, rw = e3_w;
+			e3_e = e3_ne; e3_w = e3_nw;
+			e3_load(w + 2 * gp.nw, e3_ne, e3_nw);
+			u32 V = 0;
+			if (e != 0xff) {
+				u32 step = (rw & 0x80000000u) ? (rw & 0xffff) : 1;
+				u32 j = lane + step;
+				u32 jk[5];
+#pragma unroll
+				for (int k = 0; k < 5; k++) {
+					jk[k] = j;
+					u32 t = __shfl_sync(LDB_FULL_MASK, j, j & 31);
+					if (j < 32) j = t;
+				}
+				V = 1u << e;
+#pragma unroll
+				for (int k = 4; k >= 0; k--) {
+					u32 contrib = (((V >> lane) & 1) && jk[k] < 32) ? (1u << jk[k]) : 0;
+					V |= __reduce_or_sync(LDB_FULL_MASK, contrib);
+				}
+				// positions at or beyond the end of the pass are not tokens of this block
+				const u32 wbase = pb0 + w * 32;
+				if (wbase + 32 > ppend) V &= ppend > wbase ? ((1u << (ppend - wbase)) - 1) : 0;
 			}
-			__syncthreads();		// earlier readers of escan are done
-			if (lane == 31) escan[warp] = incl;
-			__syncthreads();
-			if (warp == 0) {
-				u32 y = lane < LZ_WARPS ? escan[lane] : 0;
-				u32 yi = y;
+			if (lane == 0) vis[w] = V;
+		}
+		lz_sync(gp);
+		LZ_T(10);
+		// (e4) token offsets (exclusive scan over windows) by warp 0
+		if (gp.w == 0) {
+			u32 run = 0;
+			for (u32 w0 = 0; w0 < nwin; w0 += 32) {
+				u32 w = w0 + lane;
+				u32 c = w < nwin ? (u32)__popc(vis[w]) : 0;
+				u32 incl = c;
 				for (int o2 = 1; o2 < 32; o2 <<= 1) {
-					u32 t = __shfl_up_sync(LDB_FULL_MASK, yi, o2);
-					if (lane >= (u32)o2) yi += t;
+					u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
+					if (lane >= (u32)o2) incl += t;
 				}
-				if (lane < LZ_WARPS) escan[32 + lane] = yi - y;
-				if (lane == LZ_WARPS - 1) escan[64] = yi;
+				if (w < nwin) tokoff[w] = run + incl - c;
+				run += __shfl_sync(LDB_FULL_MASK, incl, 31);
 			}
-			__syncthreads();
-			total = escan[64];
-			return escan[32 + warp] + (incl - x);
+			if (lane == 0) tokoff[LZ_NWIN] = run;
+		}
+		lz_sync(gp);
+		LZ_T(11);
+		// (e5) emit tokens + histograms
+		const u32 tbase = v->tok_count;
+		auto e5_load = [&](u32 w, u32 &V, u32 &x) {
+			V = 0; x = 0;
+			if (w < nwin) {
+				V = vis[w];
+				if ((V >> lane) & 1) x = res[aoff + w * 32 + lane];
+			}
 		};
-		auto build_codes = [&]() {
-			// (f1) Huffman codes for both alphabets.  Parallel: rank sort by (freq, sym), leaf depths
-			// (every leaf walks to the root), length assignment, canonical codewords (rank among the
-			// symbols of equal length).  Serial: only the two-queue merges, on thread 0 (litlen)
-			// and thread 32 (offset), and the rare Kraft repair after the 15-bit cap.
-			u32 *hcount = (u32 *)(sm + LZ_SM_GEXIT + 256), *ocount = hcount + 17;	// codewords per length
-			const bool is_lit = tid < 288;
-			const u32 lo = is_lit ? 0 : 288, hi = is_lit ? 288 : 320;
-			if (tid == 0) { v->nused_lit = 0; v->nused_off = 0; v->huff_over = 0; }
-			if (tid < 34) hcount[tid] = 0;
-			__syncthreads();
-			u32 myrank = 0xffffffffu;
-			if (tid < 320) {
-				const u32 f = freq[tid];
-				lens[tid] = 0;
-				if (f) {
-					u32 rank = 0;
-					for (u32 t = lo; t < hi; t++) {
-						u32 ft = freq[t];
-						rank += (ft != 0) && (ft < f || (ft == f && t < tid));
-					}
-					myrank = rank;
-					(is_lit ? hsorted : osorted)[rank] = (u16)(tid - lo);
-					(is_lit ? hnodefreq : onodefreq)[rank] = f;
-					atomicAdd(is_lit ? &v->nused_lit : &v->nused_off, 1u);
-				}
-			}
-			__syncthreads();
-			const u32 nused = is_lit ? v->nused_lit : v->nused_off;
-			if (tid == 0 && nused >= 2) lz_huffman_merge(hnodefreq, hparent, nused);
-			if (tid == 32) { const u32 nu = v->nused_off; if (nu >= 2) lz_huffman_merge(onodefreq, oparent, nu); }
-			__syncthreads();
-			if (tid < 320 && myrank != 0xffffffffu && nused >= 2) {
-				const u16 *par = is_lit ? hparent : oparent;
-				const u32 root = 2 * nused - 2;
-				u32 node = myrank, d = 0;
-				while (node != root && d <= 15) { node = par[node]; d++; }
-				if (d > 15) { d = 15; v->huff_over = 1; }
-				atomicAdd(&(is_lit ? hcount : ocount)[d], 1u);
-			}
-			__syncthreads();
-			if ((tid == 0 || tid == 288) && nused < 2) {
-				// at least two codewords (ref: deflate_compress.c:1369-1378)
-				u8 *ln = lens + lo;
-				u32 *cn = is_lit ? hcount : ocount;
-				if (nused == 0) { ln[0] = 1; ln[1] = 1; }
-				else { const u32 sy = (is_lit ? hsorted : osorted)[0]; ln[sy] = 1; ln[sy ? 0 : 1] = 1; }
-				cn[1] = 2;
-			}
-			if ((tid == 0 || tid == 32) && v->huff_over) {
-				// restore the Kraft sum to exactly 1 by lengthening the cheapest leaves
-				u32 *cn = tid == 0 ? hcount : ocount;
-				u32 kraft = 0;
-				for (u32 l = 1; l <= 15; l++) kraft += cn[l] << (15 - l);
-				while (kraft > (1u << 15)) {
-					u32 l = 14;
-					while (cn[l] == 0) l--;
-					cn[l]--;
-					cn[l + 1] += 2;
-					cn[15]--;
-					kraft -= 1;
-				}
-			}
-			__syncthreads();
-			if (tid < 320 && myrank != 0xffffffffu && nused >= 2) {
-				// rarest symbols get the longest codes
-				const u32 *cn = is_lit ? hcount : ocount;
-				u32 cum = 0, len = 1;
-				for (u32 l = 15; l >= 1; l--) {
-					cum += cn[l];
-					if (myrank < cum) { len = l; break; }
-				}
-				lens[tid] = (u8)len;
-			}
-			__syncthreads();
-			if (tid < 320) {
-				const u32 l = lens[tid];
-				u32 code = 0;
-				if (l) {
-					const u32 *cn = is_lit ? hcount : ocount;
-					u32 first = 0;
-					for (u32 k = 1; k < l; k++) first = (first + cn[k]) << 1;
-					u32 same = 0;
-					for (u32 t = lo; t < tid; t++) same += lens[t] == l;
-					code = __brev(first + same) >> (32 - l);
-				}
-				codes[tid] = (u16)code;
-			}
-			__syncthreads();
-		};
-
-		u32 loaded_end = 0;
-		u32 block_begin = 0;
-		u32 block_entry = 0;	// position of the first token of the current block
-		u32 pass_in_block = 0;
-
-		for (u32 b0 = 0; b0 < n; b0 += LZ_PASS) {
-			const u32 pend = b0 + LZ_PASS < n ? b0 + LZ_PASS : n;
-			const bool last = pend >= n;
-			if (tid == 0) v->run_counter = 0;
-			__syncthreads();
-			// (a) window staging by the TMA engine, one pass ahead: searching this pass needs
-			// [b0 - MAX_DIST, pend + LOOKAHEAD), inserting the next one (concurrently) needs the
-			// bytes up to pend + PASS + 3.  The ring then still holds everything back to
-			// b0 - 32768 + 16, i.e. the whole MAX_DIST window.
-			{
-				const u32 want = pend + LZ_PASS + 16 < n ? pend + LZ_PASS + 16 : n;
-				while (loaded_end < want) {
-					u32 room = LZ_RING - (loaded_end & (LZ_RING - 1));	// a segment must not wrap
-					u32 to = loaded_end + (room < LZ_SEG ? room : LZ_SEG);
-					if (to > want) to = want;
-					lz_load_segment(sm, v, in, loaded_end, to);
-					loaded_end = to;
-				}
-			}
-			if (b0 == 0) {
-				// alphabet size of the first 4 KiB -> minimum match length (ref:
-				// calculate_min_match_len, lib/deflate_compress.c:2329-2346)
-				if (tid < 8) { v->used_lits[tid] = 0; v->obs_blk[tid] = 0; }
-				__syncthreads();
-				lz_observe(ring, 0, pend, v->obs_blk, tid, lane);
-				const u32 scan = n < 4096 ? n : 4096;
-				for (u32 i = tid; i < scan; i += LZ_THREADS) {
-					u32 bv = ring[i];
-					atomicOr(&v->used_lits[bv >> 5], 1u << (bv & 31));
-				}
-				__syncthreads();
-				if (tid == 0) {
-					u32 cnt = 0;
-					for (int k = 0; k < 8; k++) cnt += __popc(v->used_lits[k]);
-					v->min_len = n < 512 ? 4 : lz_choose_min_len(cnt, (u32)P.depth);
-					// few distinct byte values = cheap literals (text): a far 4-byte match loses against them
-					v->far4_dist = cnt < 80 ? LZ_FAR4_DIST : LZ_WIN;
-				}
-				__syncthreads();
-			}
-			// (b) the whole CTA links this pass into the hash chains (ordered within a hash)
-			LZ_T(0);	// loads + first-pass extras
-#ifdef LZ_TIMING
-			lz_insert_pass_par(ring, head, nextt, (u32 *)(sm + LZ_SM_R), b0, pend, n, tid, lane, warp, tacc, tlast);
-#else
-			lz_insert_pass_par(ring, head, nextt, (u32 *)(sm + LZ_SM_R), b0, pend, n, tid, lane, warp);
-#endif
-			LZ_T(3);	// insertion: linking
-			{
-				// (c) guided search.  Every searcher owns a run of consecutive positions and walks
-				// it like the reference's lazy parser (deflate_compress.c:2605-2808): search where
-				// a token could start, look one position ahead, then skip the positions the
-				// chosen match covers (they inherit it at the same distance).  Every position
-				// still gets a (length, distance), so the exact parallel parse below can start a
-				// token anywhere.  One search call site per loop trip keeps the warp converged.
-				u32 *rs = res + pass_in_block * LZ_PASS;
-				if (P.opt_iters) {
-					// levels 10-12: every position is searched and keeps its list of matches
-					for (u32 i = tid; b0 + i < pend; i += LZ_THREADS) {
-						const u32 p = b0 + i;
-						u32 L = 0, D = 0;
-						u32 *ml = mlist + (size_t)(pass_in_block * LZ_PASS + i) * LZ_OPT_K;
-						if (p + 4 <= n) {
-							lz_search_all(ring, nextt, p, n, P.depth, (u32)P.nice, ml, L, D);
-						} else {
-							for (u32 k = 0; k < LZ_OPT_K; k++) ml[k] = 0;
-						}
-						rs[i] = L ? L | ((D - 1) << 16) : 0;
-					}
+		u32 e5_V, e5_w, e5_nV, e5_nw;
+		e5_load(gp.w, e5_V, e5_w);
+		e5_load(gp.w + gp.nw, e5_nV, e5_nw);
+		for (u32 w = gp.w; w < nwin; w += gp.nw) {
+			const u32 V = e5_V, ro = e5_w >> 16;
+			const u32 len = e5_w & 0xffff;
+			e5_V = e5_nV; e5_w = e5_nw;
+			e5_load(w + 2 * gp.nw, e5_nV, e5_nw);
+			if (!V) continue;
+			u32 i = w * 32 + lane;
+			if ((V >> lane) & 1) {
+				u32 idx = tbase + tokoff[w] + __popc(V & ((1u << lane) - 1));
+				u32 off = (ro & 0x7fff) + 1;
+				// (a match that does not fit the data would be a bug upstream; never emit one)
+				if ((ro & 0x8000) && len >= 3 && len <= 258 && off <= pb0 + i && pb0 + i + len <= n) {
+					tokbuf[idx] = 0x80000000u | ((len - 3) << 15) | (off - 1);
+					atomicAdd(&freq[257 + lz_len_slot(len)], 1u);
+					atomicAdd(&freq[288 + lz_off_slot(off)], 1u);
 				} else {
-				const u32 min_len = v->min_len, far4 = v->far4_dist;
-				// A run starts its walk without knowing where the parse really enters it, so short
-				// runs cost a little ratio (L6: +0.9 % at 16 vs 32) and buy parallelism; the deep
-				// levels, which are chosen for ratio, keep 32.
+					u32 bv = lz_ld8(ring, pb0 + i);
+					tokbuf[idx] = bv;
+					atomicAdd(&freq[bv], 1u);
+				}
+			}
+		}
+		lz_sync(gp);
+		if (gp.t == 0) v->tok_count = tbase + tokoff[LZ_NWIN];
+		lz_sync(gp);
+	};
+
+	// ---- Huffman codes from freq[] -> lens[], codes[] (all threads)
+	// CTA-wide exclusive scan (all threads must call it); escan[0..64] is the scratch
+	auto cta_excl_scan = [&](const lz_grp &gp, u32 x, u32 &total) -> u32 {
+		u32 incl = x;
+		for (int o2 = 1; o2 < 32; o2 <<= 1) {
+			u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
+			if (lane >= (u32)o2) incl += t;
+		}
+		lz_sync(gp);		// earlier readers of escan are done
+		if (lane == 31) escan[gp.w] = incl;
+		lz_sync(gp);
+		if (gp.w == 0) {
+			u32 y = lane < gp.nw ? escan[lane] : 0;
+			u32 yi = y;
+			for (int o2 = 1; o2 < 32; o2 <<= 1) {
+				u32 t = __shfl_up_sync(LDB_FULL_MASK, yi, o2);
+				if (lane >= (u32)o2) yi += t;
+			}
+			if (lane < gp.nw) escan[32 + lane] = yi - y;
+			if (lane == gp.nw - 1) escan[64] = yi;
+		}
+		lz_sync(gp);
+		total = escan[64];
+		return escan[32 + gp.w] + (incl - x);
+	};
+	auto build_codes = [&](const lz_grp &gp) {
+		// (f1) Huffman codes for both alphabets.  Parallel: rank sort by (freq, sym), leaf depths
+		// (every leaf walks to the root), length assignment, canonical codewords (rank among the
+		// symbols of equal length).  Serial: only the two-queue merges, on thread 0 (litlen)
+		// and thread 32 (offset), and the rare Kraft repair after the 15-bit cap.
+		u32 *hcount = (u32 *)(sm + LZ_SM_GEXIT + 256), *ocount = hcount + 17;	// codewords per length
+		const bool is_lit = gp.t < 288;
+		const u32 lo = is_lit ? 0 : 288, hi = is_lit ? 288 : 320;
+		if (gp.t == 0) { v->nused_lit = 0; v->nused_off = 0; v->huff_over = 0; }
+		if (gp.t < 34) hcount[gp.t] = 0;
+		lz_sync(gp);
+		u32 myrank = 0xffffffffu;
+		if (gp.t < 320) {
+			const u32 f = freq[gp.t];
+			lens[gp.t] = 0;
+			if (f) {
+				u32 rank = 0;
+				for (u32 t = lo; t < hi; t++) {
+					u32 ft = freq[t];
+					rank += (ft != 0) && (ft < f || (ft == f && t < gp.t));
+				}
+				myrank = rank;
+				(is_lit ? hsorted : osorted)[rank] = (u16)(gp.t - lo);
+				(is_lit ? hnodefreq : onodefreq)[rank] = f;
+				atomicAdd(is_lit ? &v->nused_lit : &v->nused_off, 1u);
+			}
+		}
+		lz_sync(gp);
+		const u32 nused = is_lit ? v->nused_lit : v->nused_off;
+		if (gp.t == 0 && nused >= 2) lz_huffman_merge(hnodefreq, hparent, nused);
+		if (gp.t == 32) { const u32 nu = v->nused_off; if (nu >= 2) lz_huffman_merge(onodefreq, oparent, nu); }
+		lz_sync(gp);
+		if (gp.t < 320 && myrank != 0xffffffffu && nused >= 2) {
+			const u16 *par = is_lit ? hparent : oparent;
+			const u32 root = 2 * nused - 2;
+			u32 node = myrank, d = 0;
+			while (node != root && d <= 15) { node = par[node]; d++; }
+			if (d > 15) { d = 15; v->huff_over = 1; }
+			atomicAdd(&(is_lit ? hcount : ocount)[d], 1u);
+		}
+		lz_sync(gp);
+		if ((gp.t == 0 || gp.t == 288) && nused < 2) {
+			// at least two codewords (ref: deflate_compress.c:1369-1378)
+			u8 *ln = lens + lo;
+			u32 *cn = is_lit ? hcount : ocount;
+			if (nused == 0) { ln[0] = 1; ln[1] = 1; }
+			else { const u32 sy = (is_lit ? hsorted : osorted)[0]; ln[sy] = 1; ln[sy ? 0 : 1] = 1; }
+			cn[1] = 2;
+		}
+		if ((gp.t == 0 || gp.t == 32) && v->huff_over) {
+			// restore the Kraft sum to exactly 1 by lengthening the cheapest leaves
+			u32 *cn = gp.t == 0 ? hcount : ocount;
+			u32 kraft = 0;
+			for (u32 l = 1; l <= 15; l++) kraft += cn[l] << (15 - l);
+			while (kraft > (1u << 15)) {
+				u32 l = 14;
+				while (cn[l] == 0) l--;
+				cn[l]--;
+				cn[l + 1] += 2;
+				cn[15]--;
+				kraft -= 1;
+			}
+		}
+		lz_sync(gp);
+		if (gp.t < 320 && myrank != 0xffffffffu && nused >= 2) {
+			// rarest symbols get the longest codes
+			const u32 *cn = is_lit ? hcount : ocount;
+			u32 cum = 0, len = 1;
+			for (u32 l = 15; l >= 1; l--) {
+				cum += cn[l];
+				if (myrank < cum) { len = l; break; }
+			}
+			lens[gp.t] = (u8)len;
+		}
+		lz_sync(gp);
+		if (gp.t < 320) {
+			const u32 l = lens[gp.t];
+			u32 code = 0;
+			if (l) {
+				const u32 *cn = is_lit ? hcount : ocount;
+				u32 first = 0;
+				for (u32 k = 1; k < l; k++) first = (first + cn[k]) << 1;
+				u32 same = 0;
+				for (u32 t = lo; t < gp.t; t++) same += lens[t] == l;
+				code = __brev(first + same) >> (32 - l);
+			}
+			codes[gp.t] = (u16)code;
+		}
+		lz_sync(gp);
+	};
+
+	// ---- search half of pass [b0, pend) of input 'in' (n bytes): window loads, chain insertion,
+	// guided search -> res + roff.  Levels 1-9 need nothing else of the chunk.
+	u32 loaded_end = 0;
+	auto search_pass = [&](const lz_grp &gp, const u8 *in, const u32 n, const u32 b0, const u32 pend, const u32 roff) {
+		if (gp.t == 0) v->run_counter = 0;
+		lz_sync(gp);
+		// (a) window staging by the TMA engine, one pass ahead: searching this pass needs
+		// [b0 - MAX_DIST, pend + LOOKAHEAD), inserting the next one (concurrently) needs the
+		// bytes up to pend + PASS + 3.  The ring then still holds everything back to
+		// b0 - 32768 + 16, i.e. the whole MAX_DIST window.
+		{
+			const u32 want = pend + LZ_PASS + 16 < n ? pend + LZ_PASS + 16 : n;
+			while (loaded_end < want) {
+				u32 room = LZ_RING - (loaded_end & (LZ_RING - 1));	// a segment must not wrap
+				u32 to = loaded_end + (room < LZ_SEG ? room : LZ_SEG);
+				if (to > want) to = want;
+				lz_load_segment(sm, v, in, loaded_end, to, gp);
+				loaded_end = to;
+			}
+		}
+		if (b0 == 0) {
+			// alphabet size of the first 4 KiB -> minimum match length (ref:
+			// calculate_min_match_len, lib/deflate_compress.c:2329-2346)
+			if (gp.t < 8) v->used_lits[gp.t] = 0;
+			lz_sync(gp);
+			const u32 scan = n < 4096 ? n : 4096;
+			for (u32 i = gp.t; i < scan; i += gp.nt) {
+				u32 bv = ring[i];
+				atomicOr(&v->used_lits[bv >> 5], 1u << (bv & 31));
+			}
+			lz_sync(gp);
+			if (gp.t == 0) {
+				u32 cnt = 0;
+				for (int k = 0; k < 8; k++) cnt += __popc(v->used_lits[k]);
+				v->min_len = n < 512 ? 4 : lz_choose_min_len(cnt, (u32)P.depth);
+				// few distinct byte values = cheap literals (text): a far 4-byte match loses against them
+				v->far4_dist = cnt < 80 ? LZ_FAR4_DIST : LZ_WIN;
+			}
+			lz_sync(gp);
+		}
+		// (b) the group links this pass into the hash chains (ordered within a hash)
+		LZ_T(0);	// loads + first-pass extras
+#ifdef LZ_TIMING
+#define LZ_TARGS , tacc, tlast
+#else
+#define LZ_TARGS
+#endif
+		if (pipe) lz_insert_pass_par<LZ_A_WARPS>(ring, head, nextt, (u32 *)(sm + LZ_SM_CMAT), b0, pend, n, gp, lane LZ_TARGS);
+		else lz_insert_pass_par<LZ_WARPS>(ring, head, nextt, (u32 *)(sm + LZ_SM_R), b0, pend, n, gp, lane LZ_TARGS);
+#undef LZ_TARGS
+		LZ_T(3);	// insertion: linking
+		{
+			// (c) guided search.  Every searcher owns a run of consecutive positions and walks
+			// it like the reference's lazy parser (deflate_compress.c:2605-2808): search where
+			// a token could start, look one position ahead, then skip the positions the
+			// chosen match covers (they inherit it at the same distance).  Every position
+			// still gets a (length, distance), so the exact parallel parse below can start a
+			// token anywhere.  One search call site per loop trip keeps the warp converged.
+			u32 *rs = res + roff;
+			if (P.opt_iters) {
+				// levels 10-12: every position is searched and keeps its list of matches
+				for (u32 i = gp.t; b0 + i < pend; i += gp.nt) {
+					const u32 p = b0 + i;
+					u32 L = 0, D = 0;
+					u32 *ml = mlist + (size_t)(roff + i) * LZ_OPT_K;
+					if (p + 4 <= n) {
+						lz_search_all(ring, nextt, p, n, P.depth, (u32)P.nice, ml, L, D);
+					} else {
+						for (u32 k = 0; k < LZ_OPT_K; k++) ml[k] = 0;
+					}
+					rs[i] = L ? L | ((D - 1) << 16) : 0;
+				}
+			} else {
+			const u32 min_len = v->min_len, far4 = v->far4_dist;
+			// A run starts its walk without knowing where the parse really enters it, so short
+			// runs cost a little ratio (L6: +0.9 % at 16 vs 32) and buy parallelism; the deep
+			// levels, which are chosen for ratio, keep 32.
 #ifndef LZ_RUN_SHORT
 #define LZ_RUN_SHORT 16
 #endif
-				const u32 run_len = a.level >= 7 ? 32 : LZ_RUN_SHORT;
-				// runs are handed out dynamically (shared counter): lanes whose runs are cheap
-				// (long matches, few searches) take more of them, which keeps the warp busy
-				u32 i = 0, i_end = 0;
-				u32 pL = 0, pD = 0;		// pending match at position i-pending (lazy evaluation in progress)
-				u32 pending = 0;		// 0: none, 1: looking one position ahead, 2: two positions (lazy2)
+			const u32 run_len = a.level >= 7 ? 32 : LZ_RUN_SHORT;
+			// runs are handed out dynamically (shared counter): lanes whose runs are cheap
+			// (long matches, few searches) take more of them, which keeps the warp busy
+			u32 i = 0, i_end = 0;
+			u32 pL = 0, pD = 0;		// pending match at position i-pending (lazy evaluation in progress)
+			u32 pending = 0;		// 0: none, 1: looking one position ahead, 2: two positions (lazy2)
 #if LZ_QUANTUM
-				lz_walk wk;
-				wk.left = 0; wk.best_len = 0; wk.best_dist = 0; wk.cand = 0; wk.prev_dist = 0; wk.tailo = 0; wk.tailv = 0; wk.cur = 0;
-				bool in_search = false;
+			lz_walk wk;
+			wk.left = 0; wk.best_len = 0; wk.best_dist = 0; wk.cand = 0; wk.prev_dist = 0; wk.tailo = 0; wk.tailv = 0; wk.cur = 0;
+			bool in_search = false;
 #endif
-				for (;;) {
+			for (;;) {
 #if LZ_QUANTUM
-					if (!in_search) {
+				if (!in_search) {
 #endif
-					if (i >= i_end || b0 + i >= pend) {
-						const u32 r = atomicAdd(&v->run_counter, 1u);
-						i = r * run_len;
-						if (b0 + i >= pend || i >= LZ_PASS) break;
-						i_end = i + run_len;
+				if (i >= i_end || b0 + i >= pend) {
+					const u32 r = atomicAdd(&v->run_counter, 1u);
+					i = r * run_len;
+					if (b0 + i >= pend || i >= LZ_PASS) break;
+					i_end = i + run_len;
+					pending = 0;
+				}
+#if LZ_QUANTUM
+					const u32 p0 = b0 + i;
+					wk.best_len = 0; wk.best_dist = 0; wk.left = 0;
+					if (p0 + 4 <= n) {
+						u32 sL = 0, sD = 0;
+						if (pending) { sL = pL - pending >= 4 ? pL - pending : 0; sD = pD; }
+						lz_walk_setup(ring, nextt, p0, n, P.depth >> pending, (u32)P.nice, sL, sD, wk);
+					}
+					in_search = true;
+				}
+				lz_walk_steps(ring, nextt, b0 + i, n, (u32)P.nice, wk, LZ_QUANTUM);
+				if (wk.left > 0) continue;		// the others move on; this search resumes next trip
+				in_search = false;
+				const u32 p = b0 + i;
+				u32 L = wk.best_len, D = wk.best_dist;
+#else
+				const u32 p = b0 + i;
+				u32 L = 0, D = 0;
+				if (p + 4 <= n) {
+					if (pending) { L = pL - pending >= 4 ? pL - pending : 0; D = pD; }	// the pending match continues here
+					lz_search(ring, nextt, p, n, P.depth >> pending, (u32)P.nice, L, D);
+				}
+#endif
+				rs[i] = L ? L | ((D - 1) << 16) : 0;
+				u32 mpos, mL, mD;	// match to accept this trip (mL == 0: none)
+				if (pending) {
+					// ref: deflate_compress.c:2722-2725 (margin 2, one ahead), :2757-2760 (margin 6, two ahead)
+					const int margin = pending == 1 ? 2 : 6;
+					if (L >= pL && 4 * ((int)L - (int)pL) + ((int)(31 - __clz((int)pD)) - (int)(31 - __clz((int)D))) > margin) {
+						// the lookahead match is clearly better: literal(s) before i, keep looking
+						// ahead from i unless it is long enough to take at once
+						mpos = i; mL = L >= (u32)P.nice ? L : 0; mD = D;
+						if (!mL) { pL = L; pD = D; }
+						pending = mL == 0 ? 1 : 0;
+					} else if (pending == 1 && P.lazy == 2 && i + 1 < i_end && b0 + i + 1 < pend) {
+						pending = 2;
+						mpos = i; mL = 0; mD = 0;
+					} else {
+						mpos = i - pending; mL = pL; mD = pD;
 						pending = 0;
 					}
-#if LZ_QUANTUM
-						const u32 p0 = b0 + i;
-						wk.best_len = 0; wk.best_dist = 0; wk.left = 0;
-						if (p0 + 4 <= n) {
-							u32 sL = 0, sD = 0;
-							if (pending) { sL = pL - pending >= 4 ? pL - pending : 0; sD = pD; }
-							lz_walk_setup(ring, nextt, p0, n, P.depth >> pending, (u32)P.nice, sL, sD, wk);
-						}
-						in_search = true;
-					}
-					lz_walk_steps(ring, nextt, b0 + i, n, (u32)P.nice, wk, LZ_QUANTUM);
-					if (wk.left > 0) continue;		// the others move on; this search resumes next trip
-					in_search = false;
-					const u32 p = b0 + i;
-					u32 L = wk.best_len, D = wk.best_dist;
-#else
-					const u32 p = b0 + i;
-					u32 L = 0, D = 0;
-					if (p + 4 <= n) {
-						if (pending) { L = pL - pending >= 4 ? pL - pending : 0; D = pD; }	// the pending match continues here
-						lz_search(ring, nextt, p, n, P.depth >> pending, (u32)P.nice, L, D);
-					}
-#endif
-					rs[i] = L ? L | ((D - 1) << 16) : 0;
-					u32 mpos, mL, mD;	// match to accept this trip (mL == 0: none)
-					if (pending) {
-						// ref: deflate_compress.c:2722-2725 (margin 2, one ahead), :2757-2760 (margin 6, two ahead)
-						const int margin = pending == 1 ? 2 : 6;
-						if (L >= pL && 4 * ((int)L - (int)pL) + ((int)(31 - __clz((int)pD)) - (int)(31 - __clz((int)D))) > margin) {
-							// the lookahead match is clearly better: literal(s) before i, keep looking
-							// ahead from i unless it is long enough to take at once
-							mpos = i; mL = L >= (u32)P.nice ? L : 0; mD = D;
-							if (!mL) { pL = L; pD = D; }
-							pending = mL == 0 ? 1 : 0;
-						} else if (pending == 1 && P.lazy == 2 && i + 1 < i_end && b0 + i + 1 < pend) {
-							pending = 2;
-							mpos = i; mL = 0; mD = 0;
-						} else {
-							mpos = i - pending; mL = pL; mD = pD;
-							pending = 0;
-						}
-					} else if (L >= min_len && !(L == 4 && D > far4)) {
-						if (P.lazy && L < (u32)P.nice && i + 1 < i_end && b0 + i + 1 < pend) {
-							pending = 1; pL = L; pD = D;
-							mpos = i; mL = 0; mD = 0;
-						} else {
-							mpos = i; mL = L; mD = D;
-						}
-					} else {
+				} else if (L >= min_len && !(L == 4 && D > far4)) {
+					if (P.lazy && L < (u32)P.nice && i + 1 < i_end && b0 + i + 1 < pend) {
+						pending = 1; pL = L; pD = D;
 						mpos = i; mL = 0; mD = 0;
-					}
-					if (mL) {
-						// positions covered by the accepted match inherit it at the same distance;
-						// 'mend' (end of the match at that distance) only moves forward, so extending
-						// the inherited matches (needed when the match was capped at 258) is O(1) amortised
-						u32 stop = mpos + mL < i_end ? mpos + mL : i_end;
-						if (b0 + stop > pend) stop = pend - b0;
-						u32 mend = b0 + mpos + mL;
-						for (u32 k = i + 1; k < stop; k++) {
-							const u32 pk = b0 + k;
-							// (the match ended on a mismatch unless it was capped at 258 bytes)
-							if (mL == 258)
-								while (mend < n && mend - pk < 258 && lz_ld8(ring, mend) == lz_ld8(ring, mend - mD)) mend++;
-							u32 lk = mend - pk;
-							rs[k] = lk >= 4 ? lk | ((mD - 1) << 16) : 0;
-						}
-						i = mpos + mL;
 					} else {
-						i++;
+						mpos = i; mL = L; mD = D;
+					}
+				} else {
+					mpos = i; mL = 0; mD = 0;
+				}
+				if (mL) {
+					// positions covered by the accepted match inherit it at the same distance;
+					// 'mend' (end of the match at that distance) only moves forward, so extending
+					// the inherited matches (needed when the match was capped at 258) is O(1) amortised
+					u32 stop = mpos + mL < i_end ? mpos + mL : i_end;
+					if (b0 + stop > pend) stop = pend - b0;
+					u32 mend = b0 + mpos + mL;
+					for (u32 k = i + 1; k < stop; k++) {
+						const u32 pk = b0 + k;
+						// (the match ended on a mismatch unless it was capped at 258 bytes)
+						if (mL == 258)
+							while (mend < n && mend - pk < 258 && lz_ld8(ring, mend) == lz_ld8(ring, mend - mD)) mend++;
+						u32 lk = mend - pk;
+						rs[k] = lk >= 4 ? lk | ((mD - 1) << 16) : 0;
+					}
+					i = mpos + mL;
+				} else {
+					i++;
+				}
+			}
+			}	// guided search (levels 1-9)
+		}
+		lz_sync(gp);
+		LZ_T(1);	// search phase (barrier to barrier)
+	};
+
+	// ---- encode half: the block flush (Huffman codes, precode, costs, emission) of the block that ends at pend
+	auto flush_block = [&](const lz_grp &gp, const u32 pend, const bool last) {
+		const u32 npass_block = pass_in_block;
+		pass_in_block = 0;
+		const u32 block_end = pend;
+
+		// ---- levels 10-12: near-optimal parsing of the block (ref: deflate_optimize_and_flush_block,
+		// lib/deflate_compress.c:3417-3530).  Cost model = bit lengths of the Huffman codes of the
+		// previous parse; min-cost path by backward DP over independent 2048-position segments
+		// (one warp each); the resulting choices are re-parsed by the same parallel parser.
+		for (int it = 0; it < P.opt_iters; it++) {
+			if (gp.t == 0) freq[256] = 1;
+			lz_sync(gp);
+			build_codes(gp);
+			// bit costs: unused symbols get a pessimistic default (cf. deflate_compress.c:149-151)
+			for (u32 k = gp.t; k < 256 + 259 + 32; k += gp.nt) {
+				u32 c;
+				if (k < 256) {
+					c = lens[k] ? lens[k] : 13;
+				} else if (k < 256 + 259) {
+					u32 len = k - 256;
+					if (len < 3) c = 255;
+					else { u32 sl = lz_len_slot(len); c = (lens[257 + sl] ? lens[257 + sl] : 13) + lz_len_extra_bits(sl); }
+				} else {
+					u32 sl = k - 256 - 259;
+					c = (lens[288 + sl] ? lens[288 + sl] : 10) + lz_off_extra_bits(sl);
+				}
+				costtab[k] = (u8)c;
+			}
+			lz_sync(gp);
+			{
+				const u32 rel_entry = block_entry - block_begin;	// first token of the block
+				const u32 blen_pos = block_end - block_begin;
+				for (u32 seg = gp.w; seg * LZ_DP_SEG < blen_pos; seg += gp.nw) {
+					u32 s0 = seg * LZ_DP_SEG, s1 = s0 + LZ_DP_SEG < blen_pos ? s0 + LZ_DP_SEG : blen_pos;
+					if (s0 < rel_entry) s0 = rel_entry;
+					if (s0 >= s1) continue;
+					lz_dp_segment(ring, mlist, costg, res, costtab, block_begin, s0, s1, lane);
+				}
+			}
+			lz_sync(gp);
+			// re-parse the block with the chosen path
+			for (u32 k = gp.t; k < 320; k += gp.nt) freq[k] = 0;
+			if (gp.t == 0) { v->tok_count = 0; v->parse_entry = block_entry; }
+			lz_sync(gp);
+			for (u32 pp = 0; pp < npass_block; pp++) {
+				u32 pb0 = block_begin + pp * LZ_PASS;
+				u32 ppend = pb0 + LZ_PASS < block_end ? pb0 + LZ_PASS : block_end;
+				parse_pass(gp, pb0, ppend, pp * LZ_PASS, true, nextt + ((block_begin + npass_block * LZ_PASS) & 0xffff));
+			}
+		}
+		const u32 ntok = v->tok_count;
+
+		// ======================= block flush =========================================
+		LZ_T(7);	// optimal-parse iterations
+		if (gp.t == 0) freq[256] = 1;
+		lz_sync(gp);
+		build_codes(gp);
+		LZ_T(4);	// Huffman codes
+		// (f2) precode items + precode, ref: deflate_compress.c:1483-1631.  Run-length items in
+		// parallel: thread j looks at code length j of the hlit+hdist sequence, run starts are
+		// found with ballots, every start knows in closed form how many items its run becomes,
+		// a CTA scan places them.  Only the 19-symbol precode itself is built by one thread.
+		u32 *pfreq_sm = (u32 *)(sm + LZ_SM_GEXIT);		// u32[19] (region unused while flushing)
+		u8 *plens_sm = sm + LZ_SM_GEXIT + 128;			// u8[19]
+		u16 *pcodes_sm = (u16 *)(sm + LZ_SM_GEXIT + 160);	// u16[19]
+		if (gp.t == 0) {
+			u32 hlit = 288;
+			while (hlit > 257 && lens[hlit - 1] == 0) hlit--;
+			v->hlit = hlit;
+		}
+		if (gp.t == 32) {
+			u32 hdist = 32;
+			while (hdist > 1 && lens[288 + hdist - 1] == 0) hdist--;
+			v->hdist = hdist;
+		}
+		if (gp.t >= 64 && gp.t < 64 + 19) pfreq_sm[gp.t - 64] = 0;
+		lz_sync(gp);
+		{
+			const u32 hlit = v->hlit, total = hlit + v->hdist;
+			const u32 j = gp.t;
+			const bool inb = j < total;
+			const u32 val = inb ? (j < hlit ? lens[j] : lens[288 + j - hlit]) : 0xff;
+			const u32 prv = (inb && j > 0) ? (j - 1 < hlit ? lens[j - 1] : lens[288 + j - 1 - hlit]) : 0xfe;
+			const bool isstart = inb && val != prv;
+			const u32 smask = __ballot_sync(LDB_FULL_MASK, isstart);
+			if (lane == 0 && gp.w < 10) escan[66 + gp.w] = smask;
+			lz_sync(gp);
+			u32 run = 0, cnt = 0;
+			if (isstart) {
+				u32 nxt = total;
+				u32 m = lane == 31 ? 0 : (smask & ~((2u << lane) - 1));
+				if (m) nxt = gp.w * 32 + __ffs(m) - 1;
+				else {
+					for (u32 w = gp.w + 1; w < 10; w++) {
+						u32 mm = escan[66 + w];
+						if (mm) { nxt = w * 32 + __ffs(mm) - 1; break; }
 					}
 				}
-				}	// guided search (levels 1-9)
+				run = nxt - j;
+				if (val == 0) {
+					u32 rem = run % 138;
+					cnt = run / 138 + (rem >= 3 ? 1 : rem);
+				} else if (run >= 4) {
+					u32 rem = (run - 1) % 6;
+					cnt = 1 + (run - 1) / 6 + (rem >= 3 ? 1 : rem);
+				} else cnt = run;
 			}
-			__syncthreads();
-			LZ_T(1);	// search phase (barrier to barrier)
-			// (e) exact parallel parse of this pass -> tokens + histograms
-			parse_pass(b0, pend, pass_in_block * LZ_PASS, false, nextt + ((b0 + LZ_PASS) & 0xffff));
+			u32 ntot;
+			const u32 off = cta_excl_scan(gp, cnt, ntot);
+			if (isstart) {
+				u32 ni = off;
+				if (val == 0) {
+					while (run >= 11) {
+						u32 r = run < 138 ? run : 138;
+						items[ni++] = (u16)(18 | ((r - 11) << 5));
+						atomicAdd(&pfreq_sm[18], 1u);
+						run -= r;
+					}
+					if (run >= 3) {
+						items[ni++] = (u16)(17 | ((run - 3) << 5));
+						atomicAdd(&pfreq_sm[17], 1u);
+						run = 0;
+					}
+				} else if (run >= 4) {
+					items[ni++] = (u16)val;
+					atomicAdd(&pfreq_sm[val], 1u);
+					run--;
+					while (run >= 3) {
+						u32 r = run < 6 ? run : 6;
+						items[ni++] = (u16)(16 | ((r - 3) << 5));
+						atomicAdd(&pfreq_sm[16], 1u);
+						run -= r;
+					}
+				}
+				if (run) atomicAdd(&pfreq_sm[val], run);
+				while (run) { items[ni++] = (u16)val; run--; }
+			}
+			if (gp.t == 0) v->n_items = ntot;
+		}
+		lz_sync(gp);
+		if (gp.w == 0) {
+			// the 19-symbol precode, limited to 7 bits, by warp 0: lane = symbol.  Same construction
+			// as build_codes (rank sort, two-queue merge on lane 0, leaf depths, Kraft repair, lengths
+			// by rank, canonical codewords), with the counts per length packed into one u64.
+			u32 *pnodef = (u32 *)(sm + LZ_SM_GEXIT + 512);		// u32[38]
+			u16 *ppar = (u16 *)(sm + LZ_SM_GEXIT + 672);		// u16[38]
+			const u32 lt = (1u << lane) - 1;
+			const u32 f = lane < 19 ? pfreq_sm[lane] : 0;
+			const u32 usedm = __ballot_sync(LDB_FULL_MASK, f != 0);
+			const u32 nused = __popc(usedm);
+			u32 rank = 0;
+			for (u32 t = 0; t < 19; t++) {
+				const u32 ft = __shfl_sync(LDB_FULL_MASK, f, t);
+				rank += (ft != 0) && (ft < f || (ft == f && t < lane));
+			}
+			if (f) pnodef[rank] = f;
+			__syncwarp();
+			if (lane == 0 && nused >= 2) lz_huffman_merge(pnodef, ppar, nused);
+			__syncwarp();
+			u32 d = 0;
+			bool over = false;
+			if (f && nused >= 2) {
+				const u32 root = 2 * nused - 2;
+				u32 node = rank;
+				while (node != root && d <= 7) { node = ppar[node]; d++; }
+				if (d > 7) { d = 7; over = true; }
+			}
+			u64 cn = 0;		// codewords per length, 8 bits each
+			for (u32 l = 1; l <= 7; l++) cn |= (u64)__popc(__ballot_sync(LDB_FULL_MASK, d == l)) << (8 * l);
+			if (__any_sync(LDB_FULL_MASK, over)) {
+				u32 kraft = 0;
+				for (u32 l = 1; l <= 7; l++) kraft += (u32)((cn >> (8 * l)) & 0xff) << (7 - l);
+				while (kraft > (1u << 7)) {
+					u32 l = 6;
+					while (((cn >> (8 * l)) & 0xff) == 0) l--;
+					cn -= (u64)1 << (8 * l);
+					cn += (u64)2 << (8 * (l + 1));
+					cn -= (u64)1 << (8 * 7);
+					kraft -= 1;
+				}
+			}
+			u32 len = 0;
+			if (nused >= 2) {
+				if (f) {
+					u32 cum = 0;
+					len = 1;
+					for (u32 l = 7; l >= 1; l--) {
+						cum += (u32)((cn >> (8 * l)) & 0xff);
+						if (rank < cum) { len = l; break; }
+					}
+				}
+			} else {
+				// at least two codewords
+				const u32 sy = nused ? (u32)__ffs(usedm) - 1 : 0;
+				len = (lane == sy || lane == (sy ? 0u : 1u)) ? 1 : 0;
+				cn = (u64)2 << 8;
+			}
+			u32 first = 0;
+			for (u32 k = 1; k < len; k++) first = (first + (u32)((cn >> (8 * k)) & 0xff)) << 1;
+			const u32 samem = __match_any_sync(LDB_FULL_MASK, len);
+			const u32 code = len ? __brev(first + __popc(samem & lt)) >> (32 - len) : 0;
+			if (lane < 19) { plens_sm[lane] = (u8)len; pcodes_sm[lane] = (u16)code; }
+			__syncwarp();
+			const u8 perm[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
+			const u32 nzm = __ballot_sync(LDB_FULL_MASK, lane < 19 && plens_sm[perm[lane < 19 ? lane : 0]] != 0);
+			u32 hclen = nzm ? 32 - __clz(nzm) : 0;
+			if (hclen < 4) hclen = 4;
+			u32 cost = f * len + (lane == 16 ? 2 * f : lane == 17 ? 3 * f : lane == 18 ? 7 * f : 0);
+			for (int o2 = 16; o2 > 0; o2 >>= 1) cost += __shfl_xor_sync(LDB_FULL_MASK, cost, o2);
+			if (lane == 0) {
+				v->cost_dyn = cost + 3 + 5 + 5 + 4 + 3 * hclen;
+				v->hclen = hclen;
+				v->cost_static = 3;
+				v->extra_bits = 0;
+			}
+		}
+		lz_sync(gp);
+		LZ_T(5);	// precode
+		// (f3) symbol costs (ref: deflate_compress.c:1750-1808)
+		if (gp.t < 320) {
+			u32 f = freq[gp.t];
+			if (f) {
+				u32 dyn = f * lens[gp.t];
+				u32 extra = 0, st;
+				if (gp.t < 288) {
+					st = f * lz_static_litlen_len(gp.t);
+					if (gp.t >= 257) extra = f * lz_len_extra_bits(gp.t - 257);
+				} else {
+					st = f * 5;
+					extra = f * lz_off_extra_bits(gp.t - 288);
+				}
+				atomicAdd(&v->cost_dyn, dyn + extra);
+				atomicAdd(&v->cost_static, st + extra);
+			}
+		}
+		lz_sync(gp);
+		const u32 cost_dyn = v->cost_dyn, cost_static = v->cost_static;
+		// The tokens of this block cover [block_entry, parse_entry): its first token starts where the
+		// previous block's last match ended and its own last match may run past block_end.  A
+		// stored block must cover exactly the same bytes.
+		// (past the end of the input the parser's continuation point is only window-granular)
+		const u32 sbeg = block_entry, blen = (v->parse_entry < n ? v->parse_entry : n) - block_entry;
+		const u32 bitoff = (u32)(o.obit & 7);
+		const u32 stored_pieces = blen ? (blen + 65534) / 65535 : 1;
+		// first piece: 3 header bits + pad to a byte; later pieces start byte aligned
+		const u64 cost_stored = (u64)(((bitoff + 3 + 7) & ~7u) - bitoff) + 32 + (u64)8 * blen + (u64)(stored_pieces - 1) * 40;
+		u32 btype;	// ties: stored, then static, then dynamic (deflate_compress.c:1804-1808)
+		u64 best = cost_stored;
+		btype = DEFLATE_BLOCKTYPE_STORED;
+		if (cost_static < best) { best = cost_static; btype = DEFLATE_BLOCKTYPE_STATIC; }
+		if (cost_dyn < best) { best = cost_dyn; btype = DEFLATE_BLOCKTYPE_DYNAMIC; }
+		// single bounds check for the whole block (deflate_compress.c:1811-1814)
+		const u64 need_bytes = (o.obit + best + 7) / 8 + (last ? trailer : 0);
+		if (need_bytes > o.avail) {
+			if (gp.t == 0) v->failed = 1;
+			lz_sync(gp);
+			return;
+		}
+
+		// staging covers bits starting at word 'w0' of the output; word 0 is seeded with
+		// the partial word carried from the previous flush
+		u64 w0 = o.obit >> 5;
+		for (u32 k = gp.t; k < LZ_STAGE_WORDS; k += gp.nt) stage[k] = 0;
+		lz_sync(gp);
+		if (gp.t == 0) stage[0] = v->carry;
+		lz_sync(gp);
+		if (btype == DEFLATE_BLOCKTYPE_STORED) {
+			// ---- stored: header bits via staging, raw bytes straight from the input
+			u32 src = sbeg;
+			for (u32 piece = 0; piece < stored_pieces; piece++) {
+				u32 len = blen - (src - sbeg) > 65535 ? 65535 : blen - (src - sbeg);
+				bool fin = last && piece + 1 == stored_pieces;
+				if (gp.t == 0) {
+					lz_stage_or(stage, (u32)(o.obit - (w0 << 5)), fin ? 1 : 0, 3);
+					u64 ob = (o.obit + 3 + 7) & ~(u64)7;
+					lz_stage_or(stage, (u32)(ob - (w0 << 5)), (u64)len | ((u64)(~len & 0xffff) << 16), 32);
+				}
+				o.obit = ((o.obit + 3 + 7) & ~(u64)7) + 32;
+				lz_sync(gp);
+				// flush staging up to the (byte aligned) current position, byte granular
+				{
+					u64 bytes_end = o.obit >> 3, bytes_begin = w0 * 4;
+					for (u64 k = bytes_begin + gp.t; k < bytes_end; k += gp.nt) {
+						u32 rel = (u32)(k - bytes_begin);
+						o.out[k] = (u8)(stage[rel >> 2] >> (8 * (rel & 3)));
+					}
+				}
+				lz_sync(gp);
+				for (u32 k = gp.t; k < LZ_STAGE_WORDS; k += gp.nt) stage[k] = 0;
+				u8 *dst = o.out + (o.obit >> 3);
+				for (u32 k = gp.t; k < len; k += gp.nt) dst[k] = in[src + k];
+				src += len;
+				o.obit += (u64)len * 8;
+				lz_sync(gp);
+				// re-seed staging word 0 with the bytes already written in the current word
+				w0 = o.obit >> 5;
+				if (gp.t == 0) {
+					u32 nb = (u32)((o.obit >> 3) & 3);
+					u32 wv = 0;
+					for (u32 k = 0; k < nb; k++) wv |= (u32)(*(volatile u8 *)(o.out + w0 * 4 + k)) << (8 * k);
+					stage[0] = wv;
+				}
+				lz_sync(gp);
+			}
+		} else {
+			// ---- Huffman block --------------------------------------------------------
+			if (btype == DEFLATE_BLOCKTYPE_STATIC) {
+				for (u32 s = gp.t; s < 320; s += gp.nt) lens[s] = s < 288 ? (u8)lz_static_litlen_len(s) : 5;
+				lz_sync(gp);
+				if (gp.t == 0) lz_gen_codes_serial(lens, 288, codes);
+				if (gp.t == 32) lz_gen_codes_serial(lens + 288, 32, codes + 288);
+				lz_sync(gp);
+			}
+			// header: fixed fields by thread 0, the precode items by one thread each (bit offsets
+			// from a CTA scan), directly into staging
+			u32 rel;
+			{
+				const u32 rb0 = (u32)(o.obit - (w0 << 5));
+				u32 rb = rb0 + 3;
+				if (gp.t == 0) lz_stage_or(stage, rb0, (last ? 1 : 0) | (btype << 1), 3);
+				if (btype == DEFLATE_BLOCKTYPE_DYNAMIC) {
+					const u32 hclen = v->hclen, nit = v->n_items;
+					if (gp.t == 0)
+						lz_stage_or(stage, rb, (v->hlit - 257) | ((v->hdist - 1) << 5) | ((hclen - 4) << 10), 14);
+					rb += 14;
+					if (gp.t < hclen) {
+						const u8 perm[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
+						lz_stage_or(stage, rb + 3 * gp.t, plens_sm[perm[gp.t]], 3);
+					}
+					rb += 3 * hclen;
+					u32 nb = 0, bits = 0;
+					if (gp.t < nit) {
+						const u32 it = items[gp.t], sym = it & 31, ex = it >> 5;
+						const u32 pl = plens_sm[sym];
+						const u32 eb = sym == 16 ? 2 : (sym == 17 ? 3 : (sym == 18 ? 7 : 0));
+						bits = pcodes_sm[sym] | (ex << pl);
+						nb = pl + eb;
+					}
+					u32 hbits;
+					const u32 hoff = cta_excl_scan(gp, nb, hbits);
+					lz_stage_or(stage, rb + hoff, bits, nb);
+					rb += hbits;
+				}
+				rel = rb;	// bits used in staging so far (relative to word w0)
+			}
+			lz_sync(gp);
+			// token rounds: bit lengths -> exclusive scan -> OR into staging -> flush whole words
+			const u32 tpt = LZ_THREADS / gp.nt;	// tokens per thread and round
+			for (u32 t0 = 0; t0 <= ntok; t0 += gp.nt * tpt) {
+				// (the EOB symbol is token index ntok)
+				u32 mybits[LZ_TPT_MAX] = {};
+				u64 myval[LZ_TPT_MAX] = {};
+#pragma unroll
+				for (u32 r = 0; r < LZ_TPT_MAX; r++) {
+					u32 ti = t0 + gp.t * tpt + r;
+					if (r >= tpt) {
+					} else if (ti < ntok) {
+						u32 tk = tokbuf[ti];
+						if (tk & 0x80000000u) {
+							u32 len = ((tk >> 15) & 0x1ff) + 3, off = (tk & 0x7fff) + 1;
+							u32 ls = lz_len_slot(len), os = lz_off_slot(off);
+							u32 nb = lens[257 + ls];
+							u64 val = codes[257 + ls];
+							u32 leb = lz_len_extra_bits(ls);
+							val |= (u64)(len - lz_len_base(ls)) << nb;
+							nb += leb;
+							val |= (u64)codes[288 + os] << nb;
+							nb += lens[288 + os];
+							u32 oeb = lz_off_extra_bits(os);
+							val |= (u64)(off - lz_off_base(os)) << nb;
+							nb += oeb;
+							mybits[r] = nb;
+							myval[r] = val;
+						} else {
+							mybits[r] = lens[tk];
+							myval[r] = codes[tk];
+						}
+					} else if (ti == ntok) {
+						mybits[r] = lens[256];
+						myval[r] = codes[256];
+					}
+				}
+				// CTA-wide exclusive scan of the threads' bit counts
+				u32 mine = 0;
+#pragma unroll
+				for (int r = 0; r < LZ_TPT_MAX; r++) mine += mybits[r];
+				u32 incl = mine;
+				for (int o2 = 1; o2 < 32; o2 <<= 1) {
+					u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
+					if (lane >= (u32)o2) incl += t;
+				}
+				if (lane == 31) escan[gp.w] = incl;
+				lz_sync(gp);
+				if (gp.w == 0) {
+					u32 x = lane < gp.nw ? escan[lane] : 0;
+					u32 xi = x;
+					for (int o2 = 1; o2 < 32; o2 <<= 1) {
+						u32 t = __shfl_up_sync(LDB_FULL_MASK, xi, o2);
+						if (lane >= (u32)o2) xi += t;
+					}
+					if (lane < gp.nw) escan[32 + lane] = xi - x;
+					if (lane == gp.nw - 1) escan[64] = xi;
+				}
+				lz_sync(gp);
+				u32 bitpos = rel + escan[32 + gp.w] + (incl - mine);
+#pragma unroll
+				for (int r = 0; r < LZ_TPT_MAX; r++) {
+					lz_stage_or(stage, bitpos, myval[r], mybits[r]);
+					bitpos += mybits[r];
+				}
+				const u32 round_bits = escan[64];
+				lz_sync(gp);
+				rel += round_bits;
+				// flush complete words, keep the partial one as the new stage[0]
+				u32 full = rel >> 5;
+				if (full) {
+					lz_flush_words(o, stage, w0, full, gp);
+					lz_sync(gp);
+					u32 carry = stage[full];
+					lz_sync(gp);
+					for (u32 k = gp.t; k <= full && k < LZ_STAGE_WORDS; k += gp.nt) stage[k] = 0;
+					lz_sync(gp);
+					if (gp.t == 0) stage[0] = carry;
+					w0 += full;
+					rel &= 31;
+					lz_sync(gp);
+				}
+			}
+			o.obit = (w0 << 5) + rel;
+		}
+		lz_sync(gp);
+		if (gp.t == 0) v->carry = stage[0];
+		LZ_T(6);	// costs + emission
+		// ---- next block ------------------------------------------------------------
+		block_begin = block_end;
+		block_entry = v->parse_entry;
+		for (u32 i = gp.t; i < 320; i += gp.nt) freq[i] = 0;
+		if (gp.t == 0) v->tok_count = 0;
+		lz_sync(gp);
+	};
+
+	// ---- encode half: end of the chunk (final partial byte + trailer)
+	auto chunk_end = [&](const lz_grp &gp) {
+	lz_sync(gp);
+	if (v->failed) {
+		if (gp.t == 0) a.out_nbytes[c] = 0;
+		lz_sync(gp);
+		return;
+	}
+	// ---- final partial byte + trailer ------------------------------------------------
+	{
+		u64 w0 = o.obit >> 5;
+		for (u32 k = gp.t; k < LZ_STAGE_WORDS; k += gp.nt) stage[k] = 0;
+		lz_sync(gp);
+		if (gp.t == 0) stage[0] = v->carry;
+		lz_sync(gp);
+		u64 ob = (o.obit + 7) & ~(u64)7;	// pad the last byte with zero bits
+		if (gp.t == 0 && trailer) {
+			u8 t[8];
+			def_write_trailer(t, a.format, a.checksums ? a.checksums[c] : 0, n64);
+			for (u32 k = 0; k < trailer; k++) lz_stage_or(stage, (u32)(ob - (w0 << 5)) + 8 * k, t[k], 8);
+		}
+		ob += (u64)trailer * 8;
+		lz_sync(gp);
+		u64 bytes_begin = w0 * 4, bytes_end = ob >> 3;
+		for (u64 k = bytes_begin + gp.t; k < bytes_end; k += gp.nt) {
+			u32 rel = (u32)(k - bytes_begin);
+			o.out[k] = (u8)(stage[rel >> 2] >> (8 * (rel & 3)));
+		}
+		if (gp.t == 0) a.out_nbytes[c] = (size_t)(ob >> 3);
+	}
+	lz_sync(gp);
+		LZ_T(7);	// chunk prologue/epilogue
+	};
+
+	// ---- encode half of pass s: exact parallel parse -> tokens + histograms, block-split test,
+	// release of the pass (its res slot and ring bytes are free again), then the block flush if the
+	// block ends here.  exitt: 16 Ki u16 of scratch for the parse.
+	auto encode_pass = [&](const lz_grp &gp, const u32 s, const u32 b0, u16 *exitt) {
+		const u32 pend = b0 + LZ_PASS < n ? b0 + LZ_PASS : n;
+		const bool last = pend >= n;
+		bool end_now = true;
+		if (!v->failed) {
+			parse_pass(gp, b0, pend, res_off(s), false, exitt);
 			LZ_T(2);	// parse
 			// ---- block boundary: every LZ_BLOCK_PASSES passes, or at the end of the input --------
 			// A block also ends early when the bytes of the next pass look different from the block
 			// so far (the reference's block-split test, on pass granularity).
 			pass_in_block++;
 			if (!last) {
-				if (tid < 8) v->obs_next[tid] = 0;
-				__syncthreads();
-				lz_observe(ring, pend, pend + LZ_PASS < n ? pend + LZ_PASS : n, v->obs_next, tid, lane);
-				__syncthreads();
-				if (tid == 0) v->end_early = lz_should_end_block(v->obs_blk, v->obs_next, pend - block_begin) ? 1 : 0;
-				__syncthreads();
-				const bool end_now = pass_in_block == LZ_BLOCK_PASSES || v->end_early;
-				__syncthreads();
-				if (tid < 8) v->obs_blk[tid] = end_now ? v->obs_next[tid] : v->obs_blk[tid] + v->obs_next[tid];
-				if (!end_now) continue;
+				if (gp.t < 8) v->obs_next[gp.t] = 0;
+				lz_sync(gp);
+				lz_observe(ring, pend, pend + LZ_PASS < n ? pend + LZ_PASS : n, v->obs_next, gp, lane);
+				lz_sync(gp);
+				if (gp.t == 0) v->end_early = lz_should_end_block(v->obs_blk, v->obs_next, pend - block_begin) ? 1 : 0;
+				lz_sync(gp);
+				end_now = pass_in_block == LZ_BLOCK_PASSES || v->end_early;
+				lz_sync(gp);
+				if (gp.t < 8) v->obs_blk[gp.t] = end_now ? v->obs_next[gp.t] : v->obs_blk[gp.t] + v->obs_next[gp.t];
 			}
-			const u32 npass_block = pass_in_block;
-			pass_in_block = 0;
-			const u32 block_end = pend;
+		}
+		if (pipe) lz_bar_arrive(LZ_BAR_EMPTY + (s & 1), LZ_THREADS);
+		if (end_now && !v->failed) flush_block(gp, pend, last);
+		if (last) chunk_end(gp);
+	};
 
-			// ---- levels 10-12: near-optimal parsing of the block (ref: deflate_optimize_and_flush_block,
-			// lib/deflate_compress.c:3417-3530).  Cost model = bit lengths of the Huffman codes of the
-			// previous parse; min-cost path by backward DP over independent 2048-position segments
-			// (one warp each); the resulting choices are re-parsed by the same parallel parser.
-			for (int it = 0; it < P.opt_iters; it++) {
-				if (tid == 0) freq[256] = 1;
-				__syncthreads();
-				build_codes();
-				// bit costs: unused symbols get a pessimistic default (cf. deflate_compress.c:149-151)
-				for (u32 k = tid; k < 256 + 259 + 32; k += LZ_THREADS) {
-					u32 c;
-					if (k < 256) {
-						c = lens[k] ? lens[k] : 13;
-					} else if (k < 256 + 259) {
-						u32 len = k - 256;
-						if (len < 3) c = 255;
-						else { u32 sl = lz_len_slot(len); c = (lens[257 + sl] ? lens[257 + sl] : 13) + lz_len_extra_bits(sl); }
-					} else {
-						u32 sl = k - 256 - 259;
-						c = (lens[288 + sl] ? lens[288 + sl] : 10) + lz_off_extra_bits(sl);
-					}
-					costtab[k] = (u8)c;
-				}
-				__syncthreads();
-				{
-					const u32 rel_entry = block_entry - block_begin;	// first token of the block
-					const u32 blen_pos = block_end - block_begin;
-					for (u32 seg = warp; seg * LZ_DP_SEG < blen_pos; seg += LZ_WARPS) {
-						u32 s0 = seg * LZ_DP_SEG, s1 = s0 + LZ_DP_SEG < blen_pos ? s0 + LZ_DP_SEG : blen_pos;
-						if (s0 < rel_entry) s0 = rel_entry;
-						if (s0 >= s1) continue;
-						lz_dp_segment(ring, mlist, costg, res, costtab, block_begin, s0, s1, lane);
-					}
-				}
-				__syncthreads();
-				// re-parse the block with the chosen path
-				for (u32 k = tid; k < 320; k += LZ_THREADS) freq[k] = 0;
-				if (tid == 0) { v->tok_count = 0; v->parse_entry = block_entry; }
-				__syncthreads();
-				for (u32 pp = 0; pp < npass_block; pp++) {
-					u32 pb0 = block_begin + pp * LZ_PASS;
-					u32 ppend = pb0 + LZ_PASS < block_end ? pb0 + LZ_PASS : block_end;
-					parse_pass(pb0, ppend, pp * LZ_PASS, true, nextt + ((block_begin + npass_block * LZ_PASS) & 0xffff));
-				}
+	// ---- the schedule.  The search group takes chunks from the work counter and searches their passes;
+	// pass s is handed over in slot s % 2 (res, the slot_* fields).  Pipelined, the encode group follows
+	// one pass behind; serially, the whole CTA encodes each pass right after searching it.
+	if (in_a) {
+		u32 s = 0;		// passes searched by this CTA (numbered across chunks)
+		u32 released = 0;	// passes the encode group has released (pipelined)
+		u32 prev_npass = 0;	// passes of the previous chunk
+		// wait until passes [0, upto) are released
+		auto wait_released = [&](u32 upto) {
+			while (released < upto) {
+				lz_bar_sync(LZ_BAR_EMPTY + (released & 1), LZ_THREADS);
+				released++;
 			}
-			const u32 ntok = v->tok_count;
+			LZ_T(14);	// search group: waiting for the encode group
+		};
+		for (;;) {
+			if (gA.t == 0) v->chunk = atomicAdd(a.work_counter, 1u);
+			lz_sync(gA);
+			const size_t ca = v->chunk;
+			lz_sync(gA);
+			if (ca >= a.n) break;
 
-			// ======================= block flush =========================================
-			LZ_T(7);	// optimal-parse iterations
-			if (tid == 0) freq[256] = 1;
-			__syncthreads();
-			build_codes();
-			LZ_T(4);	// Huffman codes
-			// (f2) precode items + precode, ref: deflate_compress.c:1483-1631.  Run-length items in
-			// parallel: thread j looks at code length j of the hlit+hdist sequence, run starts are
-			// found with ballots, every start knows in closed form how many items its run becomes,
-			// a CTA scan places them.  Only the 19-symbol precode itself is built by one thread.
-			u32 *pfreq_sm = (u32 *)(sm + LZ_SM_GEXIT);		// u32[19] (region unused while flushing)
-			u8 *plens_sm = sm + LZ_SM_GEXIT + 128;			// u8[19]
-			u16 *pcodes_sm = (u16 *)(sm + LZ_SM_GEXIT + 160);	// u16[19]
-			if (tid == 0) {
-				u32 hlit = 288;
-				while (hlit > 257 && lens[hlit - 1] == 0) hlit--;
-				v->hlit = hlit;
-			}
-			if (tid == 32) {
-				u32 hdist = 32;
-				while (hdist > 1 && lens[288 + hdist - 1] == 0) hdist--;
-				v->hdist = hdist;
-			}
-			if (tid >= 64 && tid < 64 + 19) pfreq_sm[tid - 64] = 0;
-			__syncthreads();
+			const u8 *ain = (const u8 *)a.in_ptrs[ca];
+			const size_t an64 = a.in_nbytes[ca];
+			// ---- tiny inputs and oversize chunks take the stored path (ref: deflate_compress.c:4041-4043)
 			{
-				const u32 hlit = v->hlit, total = hlit + v->hdist;
-				const u32 j = tid;
-				const bool inb = j < total;
-				const u32 val = inb ? (j < hlit ? lens[j] : lens[288 + j - hlit]) : 0xff;
-				const u32 prv = (inb && j > 0) ? (j - 1 < hlit ? lens[j - 1] : lens[288 + j - 1 - hlit]) : 0xfe;
-				const bool isstart = inb && val != prv;
-				const u32 smask = __ballot_sync(LDB_FULL_MASK, isstart);
-				if (lane == 0 && warp < 10) escan[66 + warp] = smask;
-				__syncthreads();
-				u32 run = 0, cnt = 0;
-				if (isstart) {
-					u32 nxt = total;
-					u32 m = lane == 31 ? 0 : (smask & ~((2u << lane) - 1));
-					if (m) nxt = warp * 32 + __ffs(m) - 1;
-					else {
-						for (u32 w = warp + 1; w < 10; w++) {
-							u32 mm = escan[66 + w];
-							if (mm) { nxt = w * 32 + __ffs(mm) - 1; break; }
-						}
+				const lz_grp &gp = gA;
+				u8 *out = (u8 *)a.out_ptrs[ca];
+				const size_t avail = a.out_avail[ca];
+				const bool passthrough = an64 <= (size_t)(55 - 4 * a.level) || an64 > 0x7fff0000u;
+				bool fits = !(overhead && avail <= overhead);
+				if (passthrough || !fits) {
+					const size_t nblocks = an64 ? (an64 + 65534) / 65535 : 1;
+					fits = fits && (an64 + 5 * nblocks <= avail - overhead);
+					if (!fits) {
+						if (gp.t == 0) a.out_nbytes[ca] = 0;
+						continue;
 					}
-					run = nxt - j;
-					if (val == 0) {
-						u32 rem = run % 138;
-						cnt = run / 138 + (rem >= 3 ? 1 : rem);
-					} else if (run >= 4) {
-						u32 rem = (run - 1) % 6;
-						cnt = 1 + (run - 1) / 6 + (rem >= 3 ? 1 : rem);
-					} else cnt = run;
-				}
-				u32 ntot;
-				const u32 off = cta_excl_scan(cnt, ntot);
-				if (isstart) {
-					u32 ni = off;
-					if (val == 0) {
-						while (run >= 11) {
-							u32 r = run < 138 ? run : 138;
-							items[ni++] = (u16)(18 | ((r - 11) << 5));
-							atomicAdd(&pfreq_sm[18], 1u);
-							run -= r;
+					if (gp.t == 0) def_write_header(out, a.format, a.level);
+					u8 *dst = out + hdr_bytes;
+					for (size_t b = 0; b < nblocks; b++) {
+						size_t off = b * 65535;
+						u32 len = (u32)(an64 - off > 65535 ? 65535 : an64 - off);
+						if (gp.t == 0) {
+							dst[0] = (b + 1 == nblocks) ? 1 : 0;
+							dst[1] = (u8)len; dst[2] = (u8)(len >> 8);
+							dst[3] = (u8)~len; dst[4] = (u8)(~len >> 8);
 						}
-						if (run >= 3) {
-							items[ni++] = (u16)(17 | ((run - 3) << 5));
-							atomicAdd(&pfreq_sm[17], 1u);
-							run = 0;
-						}
-					} else if (run >= 4) {
-						items[ni++] = (u16)val;
-						atomicAdd(&pfreq_sm[val], 1u);
-						run--;
-						while (run >= 3) {
-							u32 r = run < 6 ? run : 6;
-							items[ni++] = (u16)(16 | ((r - 3) << 5));
-							atomicAdd(&pfreq_sm[16], 1u);
-							run -= r;
-						}
+						for (u32 i = gp.t; i < len; i += gp.nt) dst[5 + i] = ain[off + i];
+						dst += 5 + len;
 					}
-					if (run) atomicAdd(&pfreq_sm[val], run);
-					while (run) { items[ni++] = (u16)val; run--; }
+					if (gp.t == 0) {
+						u32 t = def_write_trailer(dst, a.format, a.checksums ? a.checksums[ca] : 0, an64);
+						a.out_nbytes[ca] = (size_t)(dst - out) + t;
+					}
+					continue;
 				}
-				if (tid == 0) v->n_items = ntot;
 			}
-			__syncthreads();
-			if (warp == 0) {
-				// the 19-symbol precode, limited to 7 bits, by warp 0: lane = symbol.  Same construction
-				// as build_codes (rank sort, two-queue merge on lane 0, leaf depths, Kraft repair, lengths
-				// by rank, canonical codewords), with the counts per length packed into one u64.
-				u32 *pnodef = (u32 *)(sm + LZ_SM_GEXIT + 512);		// u32[38]
-				u16 *ppar = (u16 *)(sm + LZ_SM_GEXIT + 672);		// u16[38]
-				const u32 lt = (1u << lane) - 1;
-				const u32 f = lane < 19 ? pfreq_sm[lane] : 0;
-				const u32 usedm = __ballot_sync(LDB_FULL_MASK, f != 0);
-				const u32 nused = __popc(usedm);
-				u32 rank = 0;
-				for (u32 t = 0; t < 19; t++) {
-					const u32 ft = __shfl_sync(LDB_FULL_MASK, f, t);
-					rank += (ft != 0) && (ft < f || (ft == f && t < lane));
+			const u32 an = (u32)an64;
+			for (u32 i = gA.t; i < (1u << LZ_HASH_BITS) / 2; i += gA.nt) ((u32 *)head)[i] = 0xffffffffu;
+			loaded_end = 0;
+			for (u32 b0 = 0; b0 < an; b0 += LZ_PASS, s++) {
+				const u32 pend = b0 + LZ_PASS < an ? b0 + LZ_PASS : an;
+				if (pipe) {
+					// Pass s reuses res slot s % 2 and, with the ring one pass ahead, overwrites the ring
+					// bytes of pass s - 3 and the first 16 of pass s - 2: pass s - 2 must be released.  The
+					// encode group then works on pass s - 1 at most, which reads the ring bytes of passes
+					// s - 1 and s.  The first pass of a chunk reloads ring slots [0, 2 PASS + 16), which the
+					// previous chunk's last pass reads unless it sat in the last quarter of the ring.
+					wait_released(s >= 1 ? s - 1 : 0);
+					if (b0 == 0 && (prev_npass & 3) != 0) wait_released(s);
 				}
-				if (f) pnodef[rank] = f;
-				__syncwarp();
-				if (lane == 0 && nused >= 2) lz_huffman_merge(pnodef, ppar, nused);
-				__syncwarp();
-				u32 d = 0;
-				bool over = false;
-				if (f && nused >= 2) {
-					const u32 root = 2 * nused - 2;
-					u32 node = rank;
-					while (node != root && d <= 7) { node = ppar[node]; d++; }
-					if (d > 7) { d = 7; over = true; }
-				}
-				u64 cn = 0;		// codewords per length, 8 bits each
-				for (u32 l = 1; l <= 7; l++) cn |= (u64)__popc(__ballot_sync(LDB_FULL_MASK, d == l)) << (8 * l);
-				if (__any_sync(LDB_FULL_MASK, over)) {
-					u32 kraft = 0;
-					for (u32 l = 1; l <= 7; l++) kraft += (u32)((cn >> (8 * l)) & 0xff) << (7 - l);
-					while (kraft > (1u << 7)) {
-						u32 l = 6;
-						while (((cn >> (8 * l)) & 0xff) == 0) l--;
-						cn -= (u64)1 << (8 * l);
-						cn += (u64)2 << (8 * (l + 1));
-						cn -= (u64)1 << (8 * 7);
-						kraft -= 1;
+				search_pass(gA, ain, an, b0, pend, res_off(s));
+				if (pipe) {
+					if (gA.t == 0) {
+						v->slot_chunk[s & 1] = (u32)ca;
+						v->slot_b0[s & 1] = b0;
+						v->slot_min_len[s & 1] = v->min_len;
+						v->slot_far4[s & 1] = v->far4_dist;
 					}
-				}
-				u32 len = 0;
-				if (nused >= 2) {
-					if (f) {
-						u32 cum = 0;
-						len = 1;
-						for (u32 l = 7; l >= 1; l--) {
-							cum += (u32)((cn >> (8 * l)) & 0xff);
-							if (rank < cum) { len = l; break; }
-						}
-					}
+					lz_bar_arrive(LZ_BAR_FULL + (s & 1), LZ_THREADS);
 				} else {
-					// at least two codewords
-					const u32 sy = nused ? (u32)__ffs(usedm) - 1 : 0;
-					len = (lane == sy || lane == (sy ? 0u : 1u)) ? 1 : 0;
-					cn = (u64)2 << 8;
-				}
-				u32 first = 0;
-				for (u32 k = 1; k < len; k++) first = (first + (u32)((cn >> (8 * k)) & 0xff)) << 1;
-				const u32 samem = __match_any_sync(LDB_FULL_MASK, len);
-				const u32 code = len ? __brev(first + __popc(samem & lt)) >> (32 - len) : 0;
-				if (lane < 19) { plens_sm[lane] = (u8)len; pcodes_sm[lane] = (u16)code; }
-				__syncwarp();
-				const u8 perm[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-				const u32 nzm = __ballot_sync(LDB_FULL_MASK, lane < 19 && plens_sm[perm[lane < 19 ? lane : 0]] != 0);
-				u32 hclen = nzm ? 32 - __clz(nzm) : 0;
-				if (hclen < 4) hclen = 4;
-				u32 cost = f * len + (lane == 16 ? 2 * f : lane == 17 ? 3 * f : lane == 18 ? 7 * f : 0);
-				for (int o2 = 16; o2 > 0; o2 >>= 1) cost += __shfl_xor_sync(LDB_FULL_MASK, cost, o2);
-				if (lane == 0) {
-					v->cost_dyn = cost + 3 + 5 + 5 + 4 + 3 * hclen;
-					v->hclen = hclen;
-					v->cost_static = 3;
-					v->extra_bits = 0;
+					if (b0 == 0) chunk_begin(gA, ca, v->min_len, v->far4_dist);
+					encode_pass(gA, s, b0, nextt + ((b0 + LZ_PASS) & 0xffff));	// the dead link slots of the next pass
 				}
 			}
-			__syncthreads();
-			LZ_T(5);	// precode
-			// (f3) symbol costs (ref: deflate_compress.c:1750-1808)
-			if (tid < 320) {
-				u32 f = freq[tid];
-				if (f) {
-					u32 dyn = f * lens[tid];
-					u32 extra = 0, st;
-					if (tid < 288) {
-						st = f * lz_static_litlen_len(tid);
-						if (tid >= 257) extra = f * lz_len_extra_bits(tid - 257);
-					} else {
-						st = f * 5;
-						extra = f * lz_off_extra_bits(tid - 288);
-					}
-					atomicAdd(&v->cost_dyn, dyn + extra);
-					atomicAdd(&v->cost_static, st + extra);
-				}
-			}
-			__syncthreads();
-			const u32 cost_dyn = v->cost_dyn, cost_static = v->cost_static;
-			// The tokens of this block cover [block_entry, parse_entry): its first token starts where the
-			// previous block's last match ended and its own last match may run past block_end.  A
-			// stored block must cover exactly the same bytes.
-			// (past the end of the input the parser's continuation point is only window-granular)
-			const u32 sbeg = block_entry, blen = (v->parse_entry < n ? v->parse_entry : n) - block_entry;
-			const u32 bitoff = (u32)(o.obit & 7);
-			const u32 stored_pieces = blen ? (blen + 65534) / 65535 : 1;
-			// first piece: 3 header bits + pad to a byte; later pieces start byte aligned
-			const u64 cost_stored = (u64)(((bitoff + 3 + 7) & ~7u) - bitoff) + 32 + (u64)8 * blen + (u64)(stored_pieces - 1) * 40;
-			u32 btype;	// ties: stored, then static, then dynamic (deflate_compress.c:1804-1808)
-			u64 best = cost_stored;
-			btype = DEFLATE_BLOCKTYPE_STORED;
-			if (cost_static < best) { best = cost_static; btype = DEFLATE_BLOCKTYPE_STATIC; }
-			if (cost_dyn < best) { best = cost_dyn; btype = DEFLATE_BLOCKTYPE_DYNAMIC; }
-			// single bounds check for the whole block (deflate_compress.c:1811-1814)
-			const u64 need_bytes = (o.obit + best + 7) / 8 + (last ? trailer : 0);
-			if (need_bytes > o.avail) {
-				if (tid == 0) v->failed = 1;
-				__syncthreads();
-				break;
-			}
-
-			// staging covers bits starting at word 'w0' of the output; word 0 is seeded with
-			// the partial word carried from the previous flush
-			u64 w0 = o.obit >> 5;
-			for (u32 k = tid; k < LZ_STAGE_WORDS; k += LZ_THREADS) stage[k] = 0;
-			__syncthreads();
-			if (tid == 0) stage[0] = v->carry;
-			__syncthreads();
-			if (btype == DEFLATE_BLOCKTYPE_STORED) {
-				// ---- stored: header bits via staging, raw bytes straight from the input
-				u32 src = sbeg;
-				for (u32 piece = 0; piece < stored_pieces; piece++) {
-					u32 len = blen - (src - sbeg) > 65535 ? 65535 : blen - (src - sbeg);
-					bool fin = last && piece + 1 == stored_pieces;
-					if (tid == 0) {
-						lz_stage_or(stage, (u32)(o.obit - (w0 << 5)), fin ? 1 : 0, 3);
-						u64 ob = (o.obit + 3 + 7) & ~(u64)7;
-						lz_stage_or(stage, (u32)(ob - (w0 << 5)), (u64)len | ((u64)(~len & 0xffff) << 16), 32);
-					}
-					o.obit = ((o.obit + 3 + 7) & ~(u64)7) + 32;
-					__syncthreads();
-					// flush staging up to the (byte aligned) current position, byte granular
-					{
-						u64 bytes_end = o.obit >> 3, bytes_begin = w0 * 4;
-						for (u64 k = bytes_begin + tid; k < bytes_end; k += LZ_THREADS) {
-							u32 rel = (u32)(k - bytes_begin);
-							o.out[k] = (u8)(stage[rel >> 2] >> (8 * (rel & 3)));
-						}
-					}
-					__syncthreads();
-					for (u32 k = tid; k < LZ_STAGE_WORDS; k += LZ_THREADS) stage[k] = 0;
-					u8 *dst = o.out + (o.obit >> 3);
-					for (u32 k = tid; k < len; k += LZ_THREADS) dst[k] = in[src + k];
-					src += len;
-					o.obit += (u64)len * 8;
-					__syncthreads();
-					// re-seed staging word 0 with the bytes already written in the current word
-					w0 = o.obit >> 5;
-					if (tid == 0) {
-						u32 nb = (u32)((o.obit >> 3) & 3);
-						u32 wv = 0;
-						for (u32 k = 0; k < nb; k++) wv |= (u32)(*(volatile u8 *)(o.out + w0 * 4 + k)) << (8 * k);
-						stage[0] = wv;
-					}
-					__syncthreads();
-				}
-			} else {
-				// ---- Huffman block --------------------------------------------------------
-				if (btype == DEFLATE_BLOCKTYPE_STATIC) {
-					for (u32 s = tid; s < 320; s += LZ_THREADS) lens[s] = s < 288 ? (u8)lz_static_litlen_len(s) : 5;
-					__syncthreads();
-					if (tid == 0) lz_gen_codes_serial(lens, 288, codes);
-					if (tid == 32) lz_gen_codes_serial(lens + 288, 32, codes + 288);
-					__syncthreads();
-				}
-				// header: fixed fields by thread 0, the precode items by one thread each (bit offsets
-				// from a CTA scan), directly into staging
-				u32 rel;
-				{
-					const u32 rb0 = (u32)(o.obit - (w0 << 5));
-					u32 rb = rb0 + 3;
-					if (tid == 0) lz_stage_or(stage, rb0, (last ? 1 : 0) | (btype << 1), 3);
-					if (btype == DEFLATE_BLOCKTYPE_DYNAMIC) {
-						const u32 hclen = v->hclen, nit = v->n_items;
-						if (tid == 0)
-							lz_stage_or(stage, rb, (v->hlit - 257) | ((v->hdist - 1) << 5) | ((hclen - 4) << 10), 14);
-						rb += 14;
-						if (tid < hclen) {
-							const u8 perm[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-							lz_stage_or(stage, rb + 3 * tid, plens_sm[perm[tid]], 3);
-						}
-						rb += 3 * hclen;
-						u32 nb = 0, bits = 0;
-						if (tid < nit) {
-							const u32 it = items[tid], sym = it & 31, ex = it >> 5;
-							const u32 pl = plens_sm[sym];
-							const u32 eb = sym == 16 ? 2 : (sym == 17 ? 3 : (sym == 18 ? 7 : 0));
-							bits = pcodes_sm[sym] | (ex << pl);
-							nb = pl + eb;
-						}
-						u32 hbits;
-						const u32 hoff = cta_excl_scan(nb, hbits);
-						lz_stage_or(stage, rb + hoff, bits, nb);
-						rb += hbits;
-					}
-					rel = rb;	// bits used in staging so far (relative to word w0)
-				}
-				__syncthreads();
-				// token rounds: bit lengths -> exclusive scan -> OR into staging -> flush whole words
-				for (u32 t0 = 0; t0 <= ntok; t0 += LZ_EMIT_ROUND) {
-					// (the EOB symbol is token index ntok)
-					u32 mybits[LZ_TPT] = {};
-					u64 myval[LZ_TPT] = {};
-#pragma unroll
-					for (int r = 0; r < LZ_TPT; r++) {
-						u32 ti = t0 + tid * LZ_TPT + r;
-						if (ti < ntok) {
-							u32 tk = tokbuf[ti];
-							if (tk & 0x80000000u) {
-								u32 len = ((tk >> 15) & 0x1ff) + 3, off = (tk & 0x7fff) + 1;
-								u32 ls = lz_len_slot(len), os = lz_off_slot(off);
-								u32 nb = lens[257 + ls];
-								u64 val = codes[257 + ls];
-								u32 leb = lz_len_extra_bits(ls);
-								val |= (u64)(len - lz_len_base(ls)) << nb;
-								nb += leb;
-								val |= (u64)codes[288 + os] << nb;
-								nb += lens[288 + os];
-								u32 oeb = lz_off_extra_bits(os);
-								val |= (u64)(off - lz_off_base(os)) << nb;
-								nb += oeb;
-								mybits[r] = nb;
-								myval[r] = val;
-							} else {
-								mybits[r] = lens[tk];
-								myval[r] = codes[tk];
-							}
-						} else if (ti == ntok) {
-							mybits[r] = lens[256];
-							myval[r] = codes[256];
-						}
-					}
-					// CTA-wide exclusive scan of the threads' bit counts
-					u32 mine = 0;
-#pragma unroll
-					for (int r = 0; r < LZ_TPT; r++) mine += mybits[r];
-					u32 incl = mine;
-					for (int o2 = 1; o2 < 32; o2 <<= 1) {
-						u32 t = __shfl_up_sync(LDB_FULL_MASK, incl, o2);
-						if (lane >= (u32)o2) incl += t;
-					}
-					if (lane == 31) escan[warp] = incl;
-					__syncthreads();
-					if (warp == 0) {
-						u32 x = lane < LZ_WARPS ? escan[lane] : 0;
-						u32 xi = x;
-						for (int o2 = 1; o2 < 32; o2 <<= 1) {
-							u32 t = __shfl_up_sync(LDB_FULL_MASK, xi, o2);
-							if (lane >= (u32)o2) xi += t;
-						}
-						if (lane < LZ_WARPS) escan[32 + lane] = xi - x;
-						if (lane == LZ_WARPS - 1) escan[64] = xi;
-					}
-					__syncthreads();
-					u32 bitpos = rel + escan[32 + warp] + (incl - mine);
-#pragma unroll
-					for (int r = 0; r < LZ_TPT; r++) {
-						lz_stage_or(stage, bitpos, myval[r], mybits[r]);
-						bitpos += mybits[r];
-					}
-					const u32 round_bits = escan[64];
-					__syncthreads();
-					rel += round_bits;
-					// flush complete words, keep the partial one as the new stage[0]
-					u32 full = rel >> 5;
-					if (full) {
-						lz_flush_words(o, stage, w0, full);
-						__syncthreads();
-						u32 carry = stage[full];
-						__syncthreads();
-						for (u32 k = tid; k <= full && k < LZ_STAGE_WORDS; k += LZ_THREADS) stage[k] = 0;
-						__syncthreads();
-						if (tid == 0) stage[0] = carry;
-						w0 += full;
-						rel &= 31;
-						__syncthreads();
-					}
-				}
-				o.obit = (w0 << 5) + rel;
-			}
-			__syncthreads();
-			if (tid == 0) v->carry = stage[0];
-			LZ_T(6);	// costs + emission
-			// ---- next block ------------------------------------------------------------
-			block_begin = block_end;
-			block_entry = v->parse_entry;
-			for (u32 i = tid; i < 320; i += LZ_THREADS) freq[i] = 0;
-			if (tid == 0) v->tok_count = 0;
-			__syncthreads();
+			prev_npass = (an + LZ_PASS - 1) / LZ_PASS;
 		}
-		__syncthreads();
-		if (v->failed) {
-			if (tid == 0) a.out_nbytes[c] = 0;
-			__syncthreads();
-			continue;
+		if (pipe) {
+			wait_released(s >= 1 ? s - 1 : 0);
+			if (gA.t == 0) v->slot_chunk[s & 1] = LZ_NO_CHUNK;
+			lz_bar_arrive(LZ_BAR_FULL + (s & 1), LZ_THREADS);
+			wait_released(s);
 		}
-		// ---- final partial byte + trailer ------------------------------------------------
-		{
-			u64 w0 = o.obit >> 5;
-			for (u32 k = tid; k < LZ_STAGE_WORDS; k += LZ_THREADS) stage[k] = 0;
-			__syncthreads();
-			if (tid == 0) stage[0] = v->carry;
-			__syncthreads();
-			u64 ob = (o.obit + 7) & ~(u64)7;	// pad the last byte with zero bits
-			if (tid == 0 && trailer) {
-				u8 t[8];
-				def_write_trailer(t, a.format, a.checksums ? a.checksums[c] : 0, n64);
-				for (u32 k = 0; k < trailer; k++) lz_stage_or(stage, (u32)(ob - (w0 << 5)) + 8 * k, t[k], 8);
-			}
-			ob += (u64)trailer * 8;
-			__syncthreads();
-			u64 bytes_begin = w0 * 4, bytes_end = ob >> 3;
-			for (u64 k = bytes_begin + tid; k < bytes_end; k += LZ_THREADS) {
-				u32 rel = (u32)(k - bytes_begin);
-				o.out[k] = (u8)(stage[rel >> 2] >> (8 * (rel & 3)));
-			}
-			if (tid == 0) a.out_nbytes[c] = (size_t)(ob >> 3);
+	} else {
+		// encode group: the parse cannot use the link slots of the next pass (the search group is
+		// inserting it), its exits go to this CTA's global scratch
+		u16 *exitg = (u16 *)(gs + LZ_GS_EXIT);
+		for (u32 s = 0;; s++) {
+			lz_bar_sync(LZ_BAR_FULL + (s & 1), LZ_THREADS);
+			LZ_T(15);	// encode group: waiting for the search group
+			const u32 cc = v->slot_chunk[s & 1];
+			if (cc == LZ_NO_CHUNK) break;
+			const u32 b0 = v->slot_b0[s & 1];
+			if (b0 == 0) chunk_begin(gB, cc, v->slot_min_len[s & 1], v->slot_far4[s & 1]);
+			encode_pass(gB, s, b0, exitg);
 		}
-		__syncthreads();
-		LZ_T(7);	// chunk prologue/epilogue
 	}
 #ifdef LZ_TIMING
-	if (tid == 0)
-		for (int k = 0; k < 15; k++) atomicAdd(&ldb_lz_timing[k], (unsigned long long)tacc[k]);
+	if (tlead)
+		for (int k = 0; k < 16; k++) atomicAdd(&ldb_lz_timing[k], (unsigned long long)tacc[k]);
 #endif
 }
 
@@ -1879,9 +2065,10 @@ extern "C" __attribute__((visibility("default"))) void ldb_lz_timing_dump(void)
 	cudaMemcpyFromSymbol(h, ldb_lz_timing, sizeof(h));
 	cudaMemcpyToSymbol(ldb_lz_timing, z, sizeof(z));
 	const char *names[16] = {"loads+first", "search phase", "parse e5", "insert: linking", "huffman", "precode", "cost+emit", "chunk pro/epilogue",
-				 "parse e1", "parse e2", "parse e3", "parse e4", "insert: hashing", "insert: slice lists", "", ""};
+				 "parse e1", "parse e2", "parse e3", "parse e4", "insert: hashing", "insert: slice lists",
+				 "search grp waits (encode)", "encode grp waits (search)"};
 	unsigned long long tot = 0;
-	for (int k = 0; k < 14; k++) tot += h[k];
+	for (int k = 0; k < 16; k++) tot += h[k];
 	for (int k = 0; k < 16; k++)
 		if (h[k]) printf("  timing %-26s %14llu cycles  %5.1f%%\n", names[k], h[k], 100.0 * (double)h[k] / (double)tot);
 }

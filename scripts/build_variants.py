@@ -25,6 +25,13 @@ VARIANTS = {
     "lit6": ["-DINF_LIT2=6"],           # up to six follow-on literals (default four)
     "g6": ["-DINF_LSUB_SM=16", "-DINF_OB=6", "-DINF_OSUB_SM=16"],      # 6-bit main offset table: more matches take the fused path
     "g6lit6": ["-DINF_LSUB_SM=16", "-DINF_OB=6", "-DINF_OSUB_SM=16", "-DINF_LIT2=6"],
+    # deflate schedule (scripts/gpu_pipeline_ab.sh): serial, and the pipeline with N search warps (default 22)
+    "ser": ["-DLZ_PIPELINE=0"],
+    "sert": ["-DLZ_PIPELINE=0", "-DLZ_TIMING"],
+    "a18": ["-DLZ_A_WARPS=18"],
+    "a20": ["-DLZ_A_WARPS=20"],
+    "a22": [],
+    "a22t": ["-DLZ_TIMING"],
 }
 # cache-streaming hints for the token stream off / 24 resolve warps per SM: no change / 10.5 ms (default 9.0)
 # decode kernel with more warps per SM (code lengths in global memory, smaller tables, register cap): 18 / 21 / 24 warps
